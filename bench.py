@@ -8,7 +8,7 @@ start ball (mcmc.py:49-51) around the published HD155358 solution, on the real H
 data-path collective in the headline loop.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--walkers 65536] [--impl reference]
-                  [--no-ess] [--no-var] [--no-sharded] [--ess-rows 2000] [--quick]
+                  [--no-ess] [--no-var] [--no-sharded] [--ess-rows 2000] [--quick] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = evaluations/s with inputs resident in HBM (CUDA events on the
 launching stream, max over ranks); `e2e` = the same through the host-buffer C-ABI call rv_loglik (pinned
@@ -23,6 +23,10 @@ host memory, H2D + D2H inside the timed region).  Beside the headline the line c
                       kernel / all-gather, host share, bit-identity against the single-GPU ensemble.
 `--impl reference` times the reference's CPU path: the oracle port of rebound's algorithm (oracle/, OpenMP over
 all host cores) on a bounded sample.
+`--dump-outputs DIR` writes what the timed path returned for its last timed step (rank 0's walkers) as DIR/logp.npy and
+DIR/status.npy (float64; logp is -inf where status != 0).  The walkers of every step come from fixed seeds, so two builds
+run with the same arguments can be compared output for output.  Above DUMP_SAMPLE walkers a fixed seeded sample of them is
+written, with their indices in DIR/walker_index.npy.
 """
 import argparse
 import json
@@ -47,6 +51,7 @@ FP10 = [0, 0, 0, 0, 0, 1, 1, 1, 1, 1]
 FE10 = [1, 2, 3, 0, 4, 1, 2, 3, 0, 4]
 EQUILIBRATED = os.path.join(ROOT, "tests", "golden", "hd155358_equilibrated_ensemble.npy")
 ROOFLINE_INPUTS = os.path.join(ROOT, "profiles", "roofline_inputs.json")     # ncu-derived figures, one file, committed
+DUMP_SAMPLE = 1 << 21         # --dump-outputs: at most this many walkers, 48 MB with their indices
 
 
 def walker_ball(W, seed):
@@ -93,6 +98,19 @@ def emit_line(line):
     else:
         sys.stdout.flush()
         os.write(_STDOUT_FD, data)
+
+
+def dump_outputs(out_dir, logp, status):
+    """--dump-outputs: one step's per-walker results as float64 .npy files; a fixed seeded sample above DUMP_SAMPLE walkers."""
+    arrays = {"logp": np.asarray(logp, dtype=np.float64), "status": np.asarray(status, dtype=np.float64)}
+    n = len(arrays["logp"])
+    if n > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+        arrays = {k: v[idx] for k, v in arrays.items()}
+        arrays["walker_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def roofline_inputs():
@@ -365,8 +383,10 @@ def run_reference(args):
     times = []
     cnt = None
     for k in range(args.steps):
-        dt, _, _, cnt = oracle_batch(obs, walker_ball(sample, 1234 + k), cores)
+        dt, logp, status, cnt = oracle_batch(obs, walker_ball(sample, 1234 + k), cores)
         times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, logp, status)
     tot = float(np.sum(times))
     value = sample * args.steps / tot
     line = {"metric": METRIC, "value": value, "unit": UNIT, "impl": "reference", "n_gpus": args.gpus, "steps": args.steps,
@@ -401,7 +421,11 @@ def main():
     ap.add_argument("--no-sharded", action="store_true", help="N > 1: skip the sharded stretch block")
     ap.add_argument("--sharded-steps", type=int, default=6)
     ap.add_argument("--quick", action="store_true", help="smoke-sized side blocks (200 ESS rows, no CPU baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write logp.npy and status.npy of the last timed step (rank 0's walkers) to DIR")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     quiet_stdout()
     if args.impl == "reference":
         run_reference(args)
@@ -433,7 +457,7 @@ def main():
     if args.mapping:
         model.set_option("mapping", args.mapping)
     W = args.walkers
-    nsets = args.steps + args.warmup
+    nsets = max(args.steps + args.warmup, 3)       # the CPU baseline below draws on sets 0, 1 and 2
     # a fresh batch of walkers for every step (global walker ids are disjoint across ranks)
     host_theta = [torch.from_numpy(walker_ball(W, 1000 * (rank + 1) + s)).pin_memory() for s in range(nsets)]
     d_theta = [t.to(dev, non_blocking=True) for t in host_theta]
@@ -477,6 +501,7 @@ def main():
         total_ms = float(t.item())
     st_np = d_status.cpu().numpy()
     ok_frac = float((st_np == 0).mean())
+    last_logp = d_logp.cpu().numpy()               # the blocks below reuse d_logp / d_status
 
     # ---- end-to-end through the host-buffer C ABI (rv_loglik): pinned host memory in, results out ----
     lib = ctx.lib
@@ -611,6 +636,8 @@ def main():
         line["var"] = var_block
     if sharded is not None:
         line["stretch_sharded"] = sharded
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_logp, st_np)
     emit_line(line)
     if world > 1:
         dist.barrier()
@@ -618,4 +645,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True                 # the benchmark leaves the tree as it found it (it may be read-only)
     main()

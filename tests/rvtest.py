@@ -24,23 +24,23 @@ _oracle_fast = None
 
 
 def oracle_fast():
-    """The oracle sources compiled -O3 -march=native ON THIS MACHINE (timing only; bench.py's CPU legs).  The file name
-    carries a tag of the host CPU's feature flags, so a build made elsewhere is never loaded; falls back to the checker
-    build if the compiler is missing."""
+    """The oracle sources compiled -O3 -march=native ON THIS MACHINE (timing only; bench.py's CPU legs).  Built afresh in a
+    temporary directory that is removed once the library is loaded, so the tree is never written (it may be read-only)
+    and a build made elsewhere or from other sources is never loaded; falls back to the checker build if the compiler is
+    missing."""
     global _oracle_fast
     if _oracle_fast is None:
-        import hashlib
+        import shutil
         import subprocess
+        import tempfile
+        tmp = tempfile.mkdtemp(prefix="rvoracle_fast_")
         try:
-            flags = [l for l in open("/proc/cpuinfo") if l.startswith("flags")][0]
-        except Exception:
-            flags = "unknown"
-        name = os.path.join("_build", "librvoracle_fast_%s.so" % hashlib.md5(flags.encode()).hexdigest()[:10])
-        path = os.path.join(ROOT, "oracle", name)
-        if not os.path.exists(path):
-            subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "fast", "FAST_OUT=" + name],
+            path = os.path.join(tmp, "librvoracle_fast.so")
+            subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "fast", "FAST_OUT=" + path],
                            capture_output=True, timeout=300)
-        _oracle_fast = C.CDLL(path) if os.path.exists(path) else oracle()
+            _oracle_fast = C.CDLL(path) if os.path.exists(path) else oracle()
+        finally:
+            shutil.rmtree(tmp, ignore_errors=True)
     return _oracle_fast
 
 
