@@ -290,8 +290,8 @@ RV_D void warp_converge() {
 #endif
 }
 
-// Per-lane store of the coefficients touched once per step: rebound's er, br (rejected-step re-prediction) and e:
-// 3*7*NC doubles, strided so that consecutive lanes touch consecutive doubles (shared memory on the device).
+// Per-lane store of the state touched once per step attempt or less (layout: Walker::SLOT_*), strided so that
+// consecutive lanes touch consecutive doubles (shared memory on the device).
 struct Hist {
     double* p;
     int stride;
@@ -315,12 +315,24 @@ struct Walker {
     static constexpr int NC = PL * D;   // coordinates held by this lane
     static_assert(PL == 1 || PL == P, "PL must be 1 or P");
 
+    // Per-lane shared-memory slots (Hist), in units of NC doubles:
+    //   [0, 21)  two banks of 7 that alternate as rebound's e and er (EBANK: which one holds e), then br[7]
+    //   21, 22, 23  x0, csx, csv: read once per accepted step (and by the encounter test), never in the loop
+    //   then four scalars, t, dt_last_done and the current hop's tmax, last_full_dt (LegCursor): read between attempts
+    // x0c = x0 - csx, v0 and a0/2 are the forms of the state the predictor-corrector loop reads; they stay in registers.
+    static constexpr int SLOT_BR = 7 * NC, SLOT_X0 = 21 * NC, SLOT_CSX = 22 * NC, SLOT_CSV = 23 * NC;
+    static constexpr int SLOT_T = 24 * NC, SLOT_DT_LAST_DONE = 24 * NC + 1, SLOT_TMAX = 24 * NC + 2, SLOT_LAST_FULL_DT = 24 * NC + 3;
+    static constexpr int STATE_DOUBLES = 24 * NC + 4;
+    static constexpr int EBANK = 14 * NC;      // the bank of e when ebank == 0 (else of er)
+
     Group<G> grp;
     Hist hist;
     // IAS15 state
-    double x0[NC], v0[NC], a0[NC], ha0[NC], csx[NC], csv[NC];
+    double x0c[NC], v0[NC], ha0[NC];   // ha0 = a0 / 2 = accel(x0) / 2
     double b[7][NC];      // b between step attempts; the g coefficients inside the predictor-corrector loop
-    double t, dt, dt_last_done;
+    double dt;
+    int ebank;            // slot of er (0 or EBANK); e is at EBANK - ebank.  An accepted step swaps the two roles
+    bool a0_stale;        // set up without its first force (accel needs the full warp; evaluated by the next attempt)
     // masses: own planets and (PL==1) the other planets in relative rank order
     double gm[PL];        // G*m of own planets
     double mu[PL];        // m/m_star of own planets
@@ -330,24 +342,47 @@ struct Walker {
     double min2;          // exit_min_distance^2
     double inv_eps;       // 1 / epsilon (the step-size controller multiplies: one IEEE division less per attempt)
     bool star_in_norm;    // sum(mu) >= 1: the star can dominate the max-norms (never for planets)
-    unsigned long long n_force, n_attempt;
+    // diagnostic work counters per item, 32 bits (fewer registers): at most 85 forces per attempt and max_attempts attempts
+    // per leg, exact for max_attempts up to 2^25 (default 2^20); larger user settings can wrap them, never the results
+    unsigned n_force, n_attempt;
+
+    RV_HD double& x0(int c) const { return hist.at(SLOT_X0 + c); }
+    RV_HD double& csx(int c) const { return hist.at(SLOT_CSX + c); }
+    RV_HD double& csv(int c) const { return hist.at(SLOT_CSV + c); }
+    RV_HD double& t() const { return hist.at(SLOT_T); }
+    RV_HD double& dt_last_done() const { return hist.at(SLOT_DT_LAST_DONE); }
+    RV_HD double& tmax() const { return hist.at(SLOT_TMAX); }
+    RV_HD double& last_full_dt() const { return hist.at(SLOT_LAST_FULL_DT); }
+
+    // PL == 1: positions of the other planets of the walker, in relative rank order (unused for PL == P)
+    using Others = double[P > 1 ? P - 1 : 1][D];
+    template <bool U>
+    RV_D void others(const double (&x)[NC], Others& xo) const {
+        if constexpr (PL == 1) {
+#pragma unroll
+            for (int o = 0; o < P - 1; o++)
+#pragma unroll
+                for (int d = 0; d < D; d++) xo[o][d] = grp.template ahead<U>(x[d], o + 1);
+        }
+    }
 
     // ---- gravity on own coordinates from positions x (own lane's coordinates) -------------------
     // Runs only inside the warp-uniform attempt body (full-mask shuffles).
     RV_D void accel(const double (&x)[NC], double (&a)[NC]) {
+        Others xo;
+        others<true>(x, xo);
+        accel(x, xo, a);
+    }
+    RV_D void accel(const double (&x)[NC], const Others& xo, double (&a)[NC]) const {
         if constexpr (PL == 1) {
             // planet - star separation ds = x + sum_j mu_j x_j = (1 + mu_own) x + sum_others mu_o x_o  (mu1 = 1 + mu_own)
-            double xo[P > 1 ? P - 1 : 1][D];
             double ds[D], r2 = 0.0;
 #pragma unroll
             for (int d = 0; d < D; d++) ds[d] = mu1 * x[d];
 #pragma unroll
             for (int o = 0; o < P - 1; o++) {
 #pragma unroll
-                for (int d = 0; d < D; d++) {
-                    xo[o][d] = grp.template ahead<true>(x[d], o + 1);
-                    ds[d] = fma(muo[o], xo[o][d], ds[d]);
-                }
+                for (int d = 0; d < D; d++) ds[d] = fma(muo[o], xo[o][d], ds[d]);
             }
 #pragma unroll
             for (int d = 0; d < D; d++) r2 = fma(ds[d], ds[d], r2);
@@ -411,32 +446,28 @@ struct Walker {
         }
     }
 
-    // reb_run_heartbeat: any pair (star included) closer than exit_min_distance?
+    // reb_run_heartbeat: any pair (star included) closer than exit_min_distance?  At positions x (others: see `others`).
     template <bool U>
-    RV_D bool encounter() const {
+    RV_D bool encounter(const double (&x)[NC], const Others& xo) const {
         bool hit = false;
         if constexpr (PL == 1) {
-            double xo[P > 1 ? P - 1 : 1][D];
             double S[D];
 #pragma unroll
-            for (int d = 0; d < D; d++) S[d] = mu[0] * x0[d];
+            for (int d = 0; d < D; d++) S[d] = mu[0] * x[d];
 #pragma unroll
             for (int o = 0; o < P - 1; o++) {
 #pragma unroll
-                for (int d = 0; d < D; d++) {
-                    xo[o][d] = grp.template ahead<U>(x0[d], o + 1);
-                    S[d] = fma(muo[o], xo[o][d], S[d]);
-                }
+                for (int d = 0; d < D; d++) S[d] = fma(muo[o], xo[o][d], S[d]);
             }
             double r2 = 0.0;
 #pragma unroll
-            for (int d = 0; d < D; d++) { const double ds = x0[d] + S[d]; r2 = fma(ds, ds, r2); }
+            for (int d = 0; d < D; d++) { const double ds = x[d] + S[d]; r2 = fma(ds, ds, r2); }
             hit = r2 < min2;
 #pragma unroll
             for (int o = 0; o < P - 1; o++) {
                 double q2 = 0.0;
 #pragma unroll
-                for (int d = 0; d < D; d++) { const double dp = x0[d] - xo[o][d]; q2 = fma(dp, dp, q2); }
+                for (int d = 0; d < D; d++) { const double dp = x[d] - xo[o][d]; q2 = fma(dp, dp, q2); }
                 hit = hit || (q2 < min2);
             }
             hit = grp.template any<U>(hit);
@@ -446,24 +477,33 @@ struct Walker {
             for (int d = 0; d < D; d++) {
                 S[d] = 0.0;
 #pragma unroll
-                for (int j = 0; j < P; j++) S[d] = fma(mu[j], x0[j * D + d], S[d]);
+                for (int j = 0; j < P; j++) S[d] = fma(mu[j], x[j * D + d], S[d]);
             }
 #pragma unroll
             for (int i = 0; i < P; i++) {
                 double r2 = 0.0;
 #pragma unroll
-                for (int d = 0; d < D; d++) { const double ds = x0[i * D + d] + S[d]; r2 = fma(ds, ds, r2); }
+                for (int d = 0; d < D; d++) { const double ds = x[i * D + d] + S[d]; r2 = fma(ds, ds, r2); }
                 hit = hit || (r2 < min2);
 #pragma unroll
                 for (int j = i + 1; j < P; j++) {
                     double q2 = 0.0;
 #pragma unroll
-                    for (int d = 0; d < D; d++) { const double dp = x0[i * D + d] - x0[j * D + d]; q2 = fma(dp, dp, q2); }
+                    for (int d = 0; d < D; d++) { const double dp = x[i * D + d] - x[j * D + d]; q2 = fma(dp, dp, q2); }
                     hit = hit || (q2 < min2);
                 }
             }
         }
         return hit && (min2 != 0.0);
+    }
+    // ... at the current position x0 (between attempts: group-mask exchanges)
+    RV_D bool encounter() const {
+        double x[NC];
+        Others xo;
+#pragma unroll
+        for (int c = 0; c < NC; c++) x[c] = x0(c);
+        others<false>(x, xo);
+        return encounter<false>(x, xo);
     }
 
     // barycentric x-velocity of the star = the RV observable (state.py:72)
@@ -530,19 +570,22 @@ struct Walker {
         for (int pl = 0; pl < PL; pl++)
 #pragma unroll
             for (int d = 0; d < D; d++) {
-                x0[pl * D + d] = xr[pl][d] - com_x[d];
+                x0(pl * D + d) = xr[pl][d] - com_x[d];
+                x0c[pl * D + d] = xr[pl][d] - com_x[d];      // x0 - csx with csx = 0
                 v0[pl * D + d] = vr[pl][d] - com_v[d];
             }
 #pragma unroll
         for (int c = 0; c < NC; c++) {
-            csx[c] = 0.0; csv[c] = 0.0; a0[c] = 0.0; ha0[c] = 0.0;
+            csx(c) = 0.0; csv(c) = 0.0; ha0[c] = 0.0;
 #pragma unroll
             for (int k = 0; k < 7; k++) {
                 b[k][c] = 0.0;
                 hist.at(k * NC + c) = 0.0; hist.at((7 + k) * NC + c) = 0.0; hist.at((14 + k) * NC + c) = 0.0;
             }
         }
-        t = 0.0; dt = md->dt0; dt_last_done = 0.0;
+        ebank = 0;
+        a0_stale = true;
+        t() = 0.0; dt = md->dt0; dt_last_done() = 0.0;
         return ST_OK;
     }
 };

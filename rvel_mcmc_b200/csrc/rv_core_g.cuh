@@ -18,17 +18,16 @@ template <int P, int D, int PL, int VAR = 0>
 struct WalkerG : Walker<P, D, PL, VAR> {
     using B = Walker<P, D, PL, VAR>;
     static constexpr int NC = B::NC;
-    static constexpr int HIST = 21;   // doubles of shared-memory history per coordinate: er[7], br[7], e[7]
-    static constexpr int DENSE0 = HIST * NC;               // then 9 per own planet: v0x, a0x, b0x..b6x of the last step
+    static constexpr int DENSE0 = B::STATE_DOUBLES;        // after Walker's slots: 9 per own planet, v0x, a0x, b0x..b6x of the last step
     static constexpr bool kDense = (VAR & 4) != 0;         // dense-output instantiation (model option dense_output)
     // off-chain sums of a substep: one accumulator (fewest FP64 instructions: +1 % in the default mode, which is bound by
     // FP64-pipe throughput) or two (shorter chains: +4 % in the dense-output mode); measured, profiles/r02p_loglik_variants.txt
     static constexpr bool kSplitAcc = kDense;
-    static constexpr int LANE_DOUBLES = HIST * NC + (kDense ? 9 * PL : 0);   // shared-memory doubles per lane
+    static constexpr int LANE_DOUBLES = DENSE0 + (kDense ? 9 * PL : 0);   // shared-memory doubles per lane
     using B::mu;
-    using B::x0; using B::v0; using B::a0; using B::ha0; using B::csx; using B::csv;
+    using B::x0c; using B::v0; using B::ha0; using B::ebank; using B::a0_stale;
     using B::b;                       // holds b between attempts and g inside the predictor-corrector loop
-    using B::t; using B::dt; using B::dt_last_done; using B::grp; using B::hist; using B::inv_eps;
+    using B::dt; using B::grp; using B::hist; using B::inv_eps;
     using B::star_in_norm; using B::n_force; using B::n_attempt;
 
     // One Gauss-Radau substep, software-pipelined: the only predictor term on the dependency chain is the one of the g
@@ -54,7 +53,7 @@ struct WalkerG : Walker<P, D, PL, VAR> {
 #pragma unroll
         for (int c = 0; c < NC; c++) {
           if constexpr (!kSplitAcc) {
-            double s0 = -a0[c] * tGA<VAR>(n);
+            double s0 = ha0[c] * (-2.0 * tGA<VAR>(n));
 #pragma unroll
             for (int i = 0; i < n - 1; i++) s0 = fma(-b[i][c], tGB<VAR>(n, i), s0);
             sc[c] = s0;
@@ -66,7 +65,7 @@ struct WalkerG : Walker<P, D, PL, VAR> {
             }
             ppn[c] = q0;
           } else {
-            double s0 = -a0[c] * tGA<VAR>(n), s1 = 0.0;
+            double s0 = ha0[c] * (-2.0 * tGA<VAR>(n)), s1 = 0.0;
 #pragma unroll
             for (int i = 0; i < n - 1; i++) {
                 if (i & 1) s1 = fma(-b[i][c], tGB<VAR>(n, i), s1);
@@ -117,7 +116,8 @@ struct WalkerG : Walker<P, D, PL, VAR> {
         return -grp.template sum<false>(s);
     }
 
-    RV_D void predict_g(double q, const double (&_e)[7], const double (&_b)[7], int c) {
+    // b of the next attempt, and its e into the slots from eo on
+    RV_D void predict_g(double q, const double (&_e)[7], const double (&_b)[7], int c, int eo) {
         // rebound: ratio > 20 -> e = b = 0.  Branch-free and select-free: q -> 0 zeroes every e, keep = 0 drops (b - e_old)
         // (for finite coefficients; a walker with non-finite coefficients is already on its way to ST_NONFINITE)
         const bool far = q > 20.0;
@@ -134,20 +134,31 @@ struct WalkerG : Walker<P, D, PL, VAR> {
 #pragma unroll
         for (int k = 0; k < 7; k++) {
             b[k][c] = fma(keep, _b[k] - _e[k], e[k]);
-            hist.at((14 + k) * NC + c) = e[k];
+            hist.at(eo + k * NC + c) = e[k];
         }
     }
 
-    // One IAS15 step attempt; same contract as Walker::attempt.
+    // One IAS15 step attempt, executed by all 32 lanes of the warp together (full-mask exchanges); `active`: this lane's
+    // group is integrating.  Returns bit 0: the step was accepted; bit 1: it was accepted and ends in an Encounter.
+    //
+    // The first force of an attempt, accel(x0), is evaluated at the end of the attempt before it: on the position the
+    // step would reach if accepted, beside the step-size controller's latency chain (group maxima, division, seventh
+    // root), and committed with the step.  A rejected step leaves x0 and so a0 as they were.  The encounter test after an
+    // accepted step reads the same positions and shares their exchange.
     RV_D int attempt(bool active) {
         warp_converge();
         if (active) { n_attempt++; }
-        this->accel(x0, a0);
-        double x0c[NC];
+        if (warp_any(a0_stale)) {          // the first attempt of an item (set up between attempts, see Walker::a0_stale)
+            double x[NC], a[NC];
+#pragma unroll
+            for (int c = 0; c < NC; c++) x[c] = this->x0(c);
+            this->accel(x, a);              // bit-identical to the a0 of the lanes that are not stale
+#pragma unroll
+            for (int c = 0; c < NC; c++) ha0[c] = 0.5 * a[c];
+            a0_stale = false;
+        }
 #pragma unroll
         for (int c = 0; c < NC; c++) {
-            ha0[c] = 0.5 * a0[c];
-            x0c[c] = x0[c] - csx[c];
             // g from b, in place (g_j needs b_k for k > j only)
 #pragma unroll
             for (int j = 0; j < 7; j++) {
@@ -160,9 +171,9 @@ struct WalkerG : Walker<P, D, PL, VAR> {
         double xp[NC], at[NC], dg6[NC], pp[NC];
 #pragma unroll
         for (int c = 0; c < NC; c++) {
-            xp[c] = x0[c]; at[c] = a0[c]; dg6[c] = 0.0;
-            // predictor partial sum of substep 1: every term but g6's (see substep_g); a0/2 joins last, so that the sums
-            // over g run while the force evaluation above is still in flight
+            // every active lane commits xp, at, dg6 in its first iteration; inactive lanes' values are never used
+            xp[c] = 0.0; at[c] = 0.0; dg6[c] = 0.0;
+            // predictor partial sum of substep 1: every term but g6's (see substep_g)
             double q0 = tPG<VAR>(1, 0) * b[0][c];
 #pragma unroll
             for (int k = 1; k < 6; k++) q0 = fma(tPG<VAR>(1, k), b[k][c], q0);
@@ -200,9 +211,9 @@ struct WalkerG : Walker<P, D, PL, VAR> {
             }
             maxdg = grp.template gmax<true>(maxdg);
             maxat = grp.template gmax<true>(maxat);
-            if (iterating) { pc_err.num = maxdg; pc_err.den = maxat; n_force += 7; }
+            if (iterating) { pc_err.num = maxdg; pc_err.den = maxat; }
         }
-        if (active) n_force += 1;
+        if (active) n_force += 7 * it + 1;
         // b from g, in place (b_k needs g_j for j > k only)
 #pragma unroll
         for (int c = 0; c < NC; c++) {
@@ -244,38 +255,43 @@ struct WalkerG : Walker<P, D, PL, VAR> {
         }
         maxak = grp.template gmax<true>(maxak);
         maxb6 = grp.template gmax<true>(maxb6);
-        // the position / velocity increments of this step (used if it is accepted): they depend on b only, so they are
-        // formed here, beside the latency chain of the step-size controller (shuffles, division, seventh root)
-        double sx[NC], sv[NC];
+        // The position this step reaches if it is accepted (compensated summation), x0c = x0 - csx there, and the force
+        // and the encounter test at it: they depend on b only, so they run beside the controller's chain below.
+        const double dt_done = dt;
+        const double dt2 = dt_done * dt_done;
+        double xn[NC], csxn[NC], an[NC];
 #pragma unroll
         for (int c = 0; c < NC; c++) {
             double s = b[6][c] * (1. / 72.);
             s = fma(b[5][c], 1. / 56., s); s = fma(b[4][c], 1. / 42., s); s = fma(b[3][c], 1. / 30., s);
             s = fma(b[2][c], 1. / 20., s); s = fma(b[1][c], 1. / 12., s); s = fma(b[0][c], 1. / 6., s);
-            sx[c] = fma(a0[c], 0.5, s);
-            double u = b[6][c] * (1. / 8.);
-            u = fma(b[5][c], 1. / 7., u); u = fma(b[4][c], 1. / 6., u); u = fma(b[3][c], 1. / 5., u);
-            u = fma(b[2][c], 1. / 4., u); u = fma(b[1][c], 1. / 3., u); u = fma(b[0][c], 1. / 2., u);
-            sv[c] = u + a0[c];
+            const double sx = ha0[c] + s;
+            const double a = this->x0(c);
+            double cs = this->csx(c) + fma(sx, dt2, v0[c] * dt_done);
+            xn[c] = a + cs;
+            csxn[c] = cs + (a - xn[c]);
         }
+        typename B::Others xo;
+        this->template others<true>(xn, xo);
+        this->accel(xn, xo, an);
+        const bool hit = this->template encounter<true>(xn, xo);
         int result = 0;
         if (active) {
             const double err = maxb6 / maxak;
-            const double dt_done = dt;
             // ratio = dt_new / dt_done as the controller produces it (rebound divides the product again; same to 1 ulp)
             double ratio = 4.0;
             if (is_normal(err)) ratio = inv_root7(err * inv_eps);
             double dt_new = ratio * dt_done;
             if (fabs(dt_new) < 0.25 * fabs(dt_done)) {
                 dt = dt_new;
-                if (dt_last_done != 0.0) {
-                    const double q = dt / dt_last_done;
+                if (this->dt_last_done() != 0.0) {
+                    const double q = dt / this->dt_last_done();
 #pragma unroll
                     for (int c = 0; c < NC; c++) {
                         double _e[7], _b[7];
 #pragma unroll
-                        for (int k = 0; k < 7; k++) { _e[k] = hist.at(k * NC + c); _b[k] = hist.at((7 + k) * NC + c); }
-                        predict_g(q, _e, _b, c);
+                        for (int k = 0; k < 7; k++) { _e[k] = hist.at(ebank + k * NC + c); _b[k] = hist.at(B::SLOT_BR + k * NC + c); }
+                        predict_g(q, _e, _b, c, B::EBANK - ebank);
                     }
                 } else {
                     // no history yet: rebound retries with the b it holds (the corrected ones)
@@ -283,49 +299,48 @@ struct WalkerG : Walker<P, D, PL, VAR> {
             } else {
                 if (fabs(dt_new) > 4.0 * fabs(dt_done)) { dt_new = dt_done * 4.0; ratio = 4.0; }   // same sign: dt_new/dt_done > 1/safety
                 dt = dt_new;
-                const double dt2 = dt_done * dt_done;
                 if constexpr (kDense) {
 #pragma unroll
                     for (int pl = 0; pl < PL; pl++) {
                         hist.at(DENSE0 + 9 * pl + 0) = v0[pl * D];
-                        hist.at(DENSE0 + 9 * pl + 1) = a0[pl * D];
+                        hist.at(DENSE0 + 9 * pl + 1) = ha0[pl * D] + ha0[pl * D];
 #pragma unroll
                         for (int k = 0; k < 7; k++) hist.at(DENSE0 + 9 * pl + 2 + k) = b[k][pl * D];
                     }
                 }
 #pragma unroll
                 for (int c = 0; c < NC; c++) {
-                    {
-                        const double a = x0[c];
-                        csx[c] += fma(sx[c], dt2, v0[c] * dt_done);
-                        x0[c] = a + csx[c];
-                        csx[c] += a - x0[c];
-                    }
-                    {
-                        const double a = v0[c];
-                        csv[c] = fma(sv[c], dt_done, csv[c]);
-                        v0[c] = a + csv[c];
-                        csv[c] += a - v0[c];
-                    }
+                    double u = b[6][c] * (1. / 8.);
+                    u = fma(b[5][c], 1. / 7., u); u = fma(b[4][c], 1. / 6., u); u = fma(b[3][c], 1. / 5., u);
+                    u = fma(b[2][c], 1. / 4., u); u = fma(b[1][c], 1. / 3., u); u = fma(b[0][c], 1. / 2., u);
+                    const double sv = u + (ha0[c] + ha0[c]);
+                    this->x0(c) = xn[c];
+                    this->csx(c) = csxn[c];
+                    x0c[c] = xn[c] - csxn[c];
+                    ha0[c] = 0.5 * an[c];
+                    const double a = v0[c];
+                    double cs = fma(sv, dt_done, this->csv(c));
+                    v0[c] = a + cs;
+                    this->csv(c) = cs + (a - v0[c]);
                 }
-                t += dt_done;
-                dt_last_done = dt_done;
+                this->t() += dt_done;
+                this->dt_last_done() = dt_done;
+                // this step's e becomes er (a swap of the two banks' roles); br is stored from the b just accepted
+                ebank = B::EBANK - ebank;
                 const double q = ratio;
 #pragma unroll
                 for (int c = 0; c < NC; c++) {
                     double _e[7], _b[7];
 #pragma unroll
                     for (int k = 0; k < 7; k++) {
-                        _e[k] = hist.at((14 + k) * NC + c); _b[k] = b[k][c];
-                        hist.at(k * NC + c) = _e[k]; hist.at((7 + k) * NC + c) = _b[k];
+                        _e[k] = hist.at(ebank + k * NC + c); _b[k] = b[k][c];
+                        hist.at(B::SLOT_BR + k * NC + c) = _b[k];
                     }
-                    predict_g(q, _e, _b, c);
+                    predict_g(q, _e, _b, c, B::EBANK - ebank);
                 }
-                result = 1;
+                result = hit ? 3 : 1;
             }
         }
-        warp_converge();
-        if (this->template encounter<true>()) result |= 2;
         return result;
     }
 

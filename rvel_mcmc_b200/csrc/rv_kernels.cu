@@ -3,8 +3,9 @@
 // loglik_kernel: persistent grid (resident CTAs x SM count); every lane group pulls (walker, leg)
 // items from a global counter and runs the IAS15 state machine of rv_loglik.cuh.  Observation epochs,
 // velocities and errors are staged once per CTA into shared memory; the once-per-step coefficients (e, and the
-// rejected-step history br/er) live in shared memory, strided per lane; x0, v0, a0, the carries and the seven g
-// coefficients per coordinate are in registers.
+// rejected-step history br/er) and the state the predictor-corrector loop never reads (x0 and the compensated-summation
+// carries) live in shared memory, strided per lane; x0 - csx, v0, a0/2 and the seven g coefficients per coordinate are in
+// registers.
 #include <cuda_runtime.h>
 #include <stdio.h>
 #include "rv_launch.h"
@@ -82,7 +83,11 @@ static cudaError_t launch_one(const LoglikArgs& a, int num_sms, cudaStream_t str
     const size_t smem_hist = sizeof(double) * (size_t)LANE_DOUBLES * NT;
     const size_t smem_obs = sizeof(double) * (size_t)3 * nobs;
     LoglikArgs args = a;
-    // stage the observations only while MINB CTAs still fit in the SM's 227 KB of shared memory
+    // stage the observations only while MINB CTAs still fit in the SM's 227 KB of shared memory.  Per lane (Walker::SLOT_*):
+    // e / er / br (21 NC doubles), x0, csx, csv (3 NC), t, dt_last_done, tmax, last_full_dt (4); + 9 per own planet in the
+    // dense-output instantiation.  The headline shape (P = 2, D = 2, one lane per planet: NC = 2) at 4 CTAs x 128 threads:
+    // 52 doubles x 8 B x 128 = 53 248 B, + 2 928 B of HD155358's 122 epochs + 1 KB reserved = 57 200 B per CTA,
+    // x 4 = 228 800 B <= 232 448 B (one double more per lane would stop the staging).
     args.stage_obs = ((smem_hist + smem_obs + 1024) * MINB <= (size_t)227 * 1024) ? 1 : 0;
     const size_t smem = smem_hist + (args.stage_obs ? smem_obs : 0);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -109,7 +114,10 @@ static cudaError_t launch_loglik_var(const LoglikArgs& a, int P, int D, int mapp
     switch (key) {
         case 120: case 121: return launch_one<1, 2, 1, 128, 3, VAR>(a, num_sms, stream);
         case 130: case 131: return launch_one<1, 3, 1, 128, 2, VAR>(a, num_sms, stream);
-        case 220: return launch_one<2, 2, 1, 128, 3, VAR>(a, num_sms, stream);
+        case 220:
+            // the headline shape: 4 CTAs x 128 threads at <= 128 registers without spills, +7 % over 3 CTAs on B200 (mapping 11)
+            if constexpr (VAR == 0) return launch_one<2, 2, 1, 128, 4, VAR>(a, num_sms, stream);
+            else return launch_one<2, 2, 1, 128, 3, VAR>(a, num_sms, stream);
         case 221: return launch_one<2, 2, 2, 128, 2, VAR>(a, num_sms, stream);
         case 230: return launch_one<2, 3, 1, 128, 2, VAR>(a, num_sms, stream);
         case 231: return launch_one<2, 3, 1, 128, 2, VAR>(a, num_sms, stream);
@@ -126,10 +134,13 @@ static cudaError_t launch_loglik_var(const LoglikArgs& a, int P, int D, int mapp
 
 cudaError_t launch_loglik(const LoglikArgs& a, int P, int D, int mapping, int dense, int num_sms, cudaStream_t stream) {
     // tuning variants of the headline instantiation (tools/bench_variants.py): model option "mapping" >= 10
-    if (P == 2 && D == 2 && mapping >= 10 && !dense) {
+    if (mapping >= 10) {
+        // the variants exist for the headline instantiation only; every other shape and the dense-output mode run the
+        // default mapping (mapping + 10 would otherwise select another shape's kernel in launch_loglik_var)
+        if (!(P == 2 && D == 2 && !dense)) return launch_loglik(a, P, D, 0, dense, num_sms, stream);
         switch (mapping) {
             case 10: return launch_one<2, 2, 1, 128, 3, 2>(a, num_sms, stream);     // IAS15 tables from the constant bank
-            case 11: return launch_one<2, 2, 1, 128, 4, 0>(a, num_sms, stream);     // 4 CTAs per SM (<= 128 registers)
+            case 11: return launch_one<2, 2, 1, 128, 3, 0>(a, num_sms, stream);     // 3 CTAs per SM (the default up to round 2)
             case 12: return launch_one<2, 2, 1, 128, 4, 2>(a, num_sms, stream);
             case 13: return launch_one<2, 2, 1, 256, 2, 0>(a, num_sms, stream);     // 2 CTAs x 256 threads (<= 128 registers)
             default: return cudaErrorInvalidValue;

@@ -37,6 +37,9 @@ struct LoglikArgs {
 
 enum : int { PH_NEED_ITEM = 0, PH_ENTRY, PH_CHECK, PH_STEP, PH_DONE };
 
+// the integration clock as check_exit reads it (it changes dt only)
+struct Clock { double t, dt, dt_last_done; };
+
 // Fetch / WarpAll are policy objects: device = atomicAdd + shuffle / __all_sync, host mirror = trivial.
 template <class WK, class Fetch, class WarpAll>
 RV_D void run_items(WK& w, const LoglikArgs& a, const double* st, const double* srv,
@@ -52,7 +55,8 @@ RV_D void run_items(WK& w, const LoglikArgs& a, const double* st, const double* 
     bool rev = false;       // this item visits its epochs in reversed storage order
     int phase = lane_active ? PH_NEED_ITEM : PH_DONE;
     long long item = -1, wi = 0, slot = 0;   // slot: where this item's partial results go (leg * W + walker)
-    const double *lt = nullptr, *lrv = nullptr, *lerr = nullptr;
+    const double* lt = nullptr;              // the leg's epochs; its velocities and errors are srv / serr from index lo
+    int lo = 0;
     LegCursor c;
     c.status = RUN; c.ie = 0; c.n = 0; c.attempts = 0; c.tmax = 0.0; c.last_full_dt = 0.0; c.chi2 = 0.0;
 
@@ -78,13 +82,13 @@ RV_D void run_items(WK& w, const LoglikArgs& a, const double* st, const double* 
                 item = fetch(w.grp);
                 if (item >= n_items) { phase = PH_DONE; break; }
                 if (curve) {
-                    wi = item; slot = item; lt = a.times; lrv = nullptr; lerr = nullptr; c.n = a.nt; rev = false;
+                    wi = item; slot = item; lt = a.times; lo = 0; c.n = a.nt; rev = false;
                 } else if (item < a.W) {       // backward legs first: they are the longer ones
                     wi = a.order ? (long long)a.order[item] : item; slot = wi;
-                    lt = st + a.nf; lrv = srv + a.nf; lerr = serr + a.nf; c.n = a.nb; rev = mono;
+                    lt = st + a.nf; lo = a.nf; c.n = a.nb; rev = mono;
                 } else {
                     wi = a.order ? (long long)a.order[item - a.W] : item - a.W; slot = a.W + wi;
-                    lt = st; lrv = srv; lerr = serr; c.n = a.nf; rev = false;
+                    lt = st; lo = 0; c.n = a.nf; rev = false;
                 }
                 w.n_force = 0; w.n_attempt = 0;
                 c.ie = 0; c.chi2 = 0.0; c.attempts = 0;
@@ -95,15 +99,15 @@ RV_D void run_items(WK& w, const LoglikArgs& a, const double* st, const double* 
                     // one integration per leg: natural steps away from t = 0, RVs read inside the steps
                     sgn = (item < a.W) ? -1.0 : 1.0;
                     w.dt = sgn * fabs(w.dt);
-                    if (w.template encounter<false>()) { finish(ST_ENCOUNTER); continue; }
+                    if (w.encounter()) { finish(ST_ENCOUNTER); continue; }
                     int st0 = ST_OK;
                     while (c.ie < c.n) {            // epochs at the start time itself (obs.tf[0] = 0, obs.tb[-1] = 0)
                         const int io = rev ? c.n - 1 - c.ie : c.ie;
-                        const double d = (lt[io] - w.t) * sgn;
+                        const double d = (lt[io] - w.t()) * sgn;
                         if (d > 0.0) break;
                         if (d < 0.0) { st0 = ST_NONFINITE; break; }       // an epoch behind the start: not a monotone leg
                         const double vx = w.star_vx();
-                        const double r = vx - lrv[io], er = lerr[io];
+                        const double r = vx - srv[lo + io], er = serr[lo + io];
                         c.chi2 += (r * r) / (er * er);
                         c.ie++;
                     }
@@ -114,15 +118,20 @@ RV_D void run_items(WK& w, const LoglikArgs& a, const double* st, const double* 
             }
             if (phase == PH_ENTRY) {            // sim.integrate(t) entry (rebound: reb_integrate)
                 if (c.ie == c.n) { finish(ST_OK); continue; }
-                c.tmax = lt[rev ? c.n - 1 - c.ie : c.ie];
-                c.last_full_dt = w.dt;
-                w.dt_last_done = 0.0;
+                w.tmax() = lt[rev ? c.n - 1 - c.ie : c.ie];
+                w.last_full_dt() = w.dt;
+                w.dt_last_done() = 0.0;
                 c.status = RUN;
-                if (w.template encounter<false>()) c.status = ST_ENCOUNTER;
+                if (w.encounter()) c.status = ST_ENCOUNTER;
                 phase = PH_CHECK;
             }
             if (phase == PH_CHECK) {
-                const int s = check_exit(w, c);
+                // the clock and the hop's tmax / last_full_dt live in shared memory (Walker::SLOT_T ...)
+                Clock k{w.t(), w.dt, w.dt_last_done()};
+                c.tmax = w.tmax(); c.last_full_dt = w.last_full_dt();
+                const int s = check_exit(k, c);
+                w.dt = k.dt;
+                w.last_full_dt() = c.last_full_dt;
                 if (s < 0) { phase = PH_STEP; break; }
                 w.dt = c.last_full_dt;
                 if (s != ST_OK) { finish(s); continue; }
@@ -132,7 +141,7 @@ RV_D void run_items(WK& w, const LoglikArgs& a, const double* st, const double* 
                     if (leader) a.rv_out[wi * a.nt + c.ie] = vx;
                 } else {
                     const int io = rev ? c.n - 1 - c.ie : c.ie;
-                    const double r = vx - lrv[io], er = lerr[io];
+                    const double r = vx - srv[lo + io], er = serr[lo + io];
                     c.chi2 += (r * r) / (er * er);
                 }
                 c.ie++;
@@ -149,16 +158,16 @@ RV_D void run_items(WK& w, const LoglikArgs& a, const double* st, const double* 
                 finish(ST_NONFINITE);
             } else if ((r & 1) && dense_mode) {
                 // epochs inside the step just accepted: (t - dt_done, t]
-                const double dt_done = w.dt_last_done;
+                const double dt_done = w.dt_last_done();
                 int st1 = (r & 2) ? ST_ENCOUNTER : ST_OK;
                 while (st1 == ST_OK && c.ie < c.n) {
                     const int io = rev ? c.n - 1 - c.ie : c.ie;
-                    if ((lt[io] - w.t) * sgn > 0.0) break;
-                    const double h = 1.0 + (lt[io] - w.t) / dt_done;
+                    if ((lt[io] - w.t()) * sgn > 0.0) break;
+                    const double h = 1.0 + (lt[io] - w.t()) / dt_done;
                     double vx = 0.0;
                     if constexpr (WK::kDense) vx = w.dense_star_vx(h, dt_done);
                     if (!isfinite(vx)) { st1 = ST_NONFINITE; break; }
-                    const double rr = vx - lrv[io], er = lerr[io];
+                    const double rr = vx - srv[lo + io], er = serr[lo + io];
                     c.chi2 += (rr * rr) / (er * er);
                     c.ie++;
                 }

@@ -1,6 +1,8 @@
 #!/usr/bin/env python3
 """Times tuning variants of the plain log-likelihood kernel (model option "mapping" >= 10, see rv_kernels.cu)
-on the bench workload (HD155358 ball, 65536 walkers).  Usage: python tools/bench_variants.py 0 1 10 11 ..."""
+on the bench workload (HD155358 ball, 65536 walkers).  Usage: python tools/bench_variants.py 0 1 10 11 ...
+0: default (4 CTAs x 128 threads), 1: thread per walker, 10: IAS15 tables from the constant bank, 11: 3 CTAs x 128 threads,
+12: 4 x 128 with the constant-bank tables, 13: 2 CTAs x 256 threads."""
 import os
 import sys
 import numpy as np
