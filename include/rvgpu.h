@@ -41,6 +41,13 @@ typedef struct rv_model rv_model; /* parameter schema resident in HBM (state.py:
 #define RV_NONFINITE   8   /* non-finite state or step-count bound hit                             */
 #define RV_NOT_SPD     9   /* SMALA metric not positive definite (mcmc.py:179-183 quits)           */
 
+/* per-walker fit code of rv_map_fit */
+#define RV_FIT_CONVERGED 0 /* Newton decrement / 2 <= tol and -H positive definite (min eigenvalue > 1e-12 max |eigenvalue|) */
+#define RV_FIT_MAXITER   1 /* max_iter accepted steps, not converged                                  */
+#define RV_FIT_STALLED   2 /* the line search found no ascent up to damping 1, or an evaluation after a step failed (status says why) */
+#define RV_FIT_SADDLE    3 /* decrement / 2 <= tol but -H not positive definite: a saddle or a direction the data do not constrain */
+#define RV_FIT_NOSTART   4 /* the start does not evaluate (status: RV_PRIOR, RV_ENCOUNTER, RV_NONFINITE); theta unchanged */
+
 /* element slots */
 #define RV_EL_M 0
 #define RV_EL_A 1
@@ -132,6 +139,21 @@ int rv_loglik_d_dd_opt(rv_ctx* ctx, const rv_model* model, const rv_obs* obs, co
 /* Same with DEVICE buffers, asynchronous on `stream`. */
 int rv_loglik_d_dd_dev(rv_ctx* ctx, const rv_model* model, const rv_obs* obs, const double* d_theta, int64_t W,
                        double* d_logp, double* d_grad, double* d_hess, int32_t* d_status, void* stream);
+
+/* ---- maximum-likelihood fit from W starts (no reference counterpart; DESIGN.md 3.6) ------------------------------- */
+/* theta[W][nvars]: starts in, optima out.  Per walker, damped saddle-free Newton: the eigen-decomposition of -H gives
+ * d = Q diag(1/lam~) Q^T g with lam~ = max(|lam|, 1e-12 lam_max) + mu lam_max; the walker stops when the Newton decrement
+ * g^T d (mu = 0) halved is <= tol.  Otherwise n_trial rows theta + 2^-j d (j < n_trial) and theta itself are evaluated by
+ * the plain likelihood in one launch; the best row with status RV_OK is taken if its logp exceeds theta's (damping
+ * mu /= 10, 0 below 1e-6), else mu = max(10 mu, 1e-6) and the walker retries from the same point (RV_FIT_STALLED once
+ * mu > 1).  damping0 is every walker's starting mu.  Derivatives come from the variational path with the hard prior
+ * tested (as rv_smala_run).  Out: logp[W], status[W], grad[W][nvars] and hess[W][nvars][nvars] (optional, NULL to skip)
+ * at the returned theta -- -inv(hess) is the Laplace covariance -- fit_code[W] (RV_FIT_*) and n_iter[W] (accepted
+ * steps).  A walker's results depend on its start only, not on W or its position.  n_trial 1..16, max_iter >= 0
+ * (0: the evaluation at the start), tol >= 0, damping0 >= 0; -30 / -31 as rv_loglik_d_dd.                          */
+int rv_map_fit(rv_ctx* ctx, const rv_model* model, const rv_obs* obs, double* theta, int64_t W, int max_iter, int n_trial,
+               double tol, double damping0, double* logp, double* grad, double* hess, int32_t* status, int32_t* fit_code,
+               int32_t* n_iter);
 
 /* ---- Mh.step (mcmc.py:107-121) for W independent chains, nsteps steps, device-resident ---------- */
 /* theta[W][nvars], logp[W]: start state in, final state out (have_logp = 0: logp is computed first, as

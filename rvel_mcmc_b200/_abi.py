@@ -13,6 +13,7 @@ import weakref
 import numpy as np
 
 RV_OK, RV_PRIOR, RV_ENCOUNTER, RV_NONFINITE, RV_NOT_SPD = 0, 1, 3, 8, 9
+RV_FIT_CONVERGED, RV_FIT_MAXITER, RV_FIT_STALLED, RV_FIT_SADDLE, RV_FIT_NOSTART = 0, 1, 2, 3, 4   # rv_map_fit fit codes
 ELEMS = ("m", "a", "h", "k", "l", "ix", "iy")       # ABI slot order (RV_EL_*)
 MAX_PLANETS = 5          # RV_MAX_PLANETS (plain likelihood, MH, stretch, WHFast)
 MAX_PLANETS_VAR = 5      # RV_MAX_PLANETS_VAR (gradient + Hessian, SMALA)
@@ -57,6 +58,8 @@ _SIGNATURES = {
                                      C.c_void_p, C.c_void_p, C.c_void_p]),
     "rv_loglik_d_dd_dev": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
                                      C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rv_map_fit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_double,
+                             C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rv_initial_conditions": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "rv_rv_curve": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_void_p,
                               C.c_void_p]),
@@ -342,6 +345,23 @@ class ModelHandle(_Handle):
                                                        C.c_void_p(d_logp), C.c_void_p(d_grad), C.c_void_p(d_hess),
                                                        C.c_void_p(d_status), C.c_void_p(stream) if stream else None),
                        "rv_loglik_d_dd_dev")
+
+    def map_fit(self, obs, theta, max_iter=50, n_trial=8, tol=1e-10, damping=0.0):
+        """Maximum-likelihood fit from every row of theta[W][nvars] (rv_map_fit: damped saddle-free Newton, batched line
+        search).  Returns dict(theta, logp, grad, hess, status, fit_code, n_iter), per walker; -inv(hess) at a converged
+        walker (fit_code RV_FIT_CONVERGED) is its Laplace covariance."""
+        theta = self._theta(theta).copy()
+        W = theta.shape[0]
+        logp = np.zeros(W)
+        grad = np.zeros((W, self.nvars))
+        hess = np.zeros((W, self.nvars, self.nvars))
+        status = np.zeros(W, dtype=np.int32)
+        code = np.zeros(W, dtype=np.int32)
+        n_iter = np.zeros(W, dtype=np.int32)
+        self.ctx.check(self.ctx.lib.rv_map_fit(self.ctx.h, self.h, obs.h, _ptr(theta), W, int(max_iter), int(n_trial),
+                                               float(tol), float(damping), _ptr(logp), _ptr(grad), _ptr(hess), _ptr(status),
+                                               _ptr(code), _ptr(n_iter)), "rv_map_fit")
+        return dict(theta=theta, logp=logp, grad=grad, hess=hess, status=status, fit_code=code, n_iter=n_iter)
 
     def initial_conditions(self, theta):
         """theta[W][nvars] -> (particles[W][P+1][7] = m,x,y,z,vx,vy,vz in the barycentric frame, status[W]);

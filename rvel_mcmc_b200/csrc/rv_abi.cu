@@ -9,6 +9,7 @@
 #include "rv_loglik.cuh"
 #include "rv_model.h"
 #include "rv_var.cuh"
+#include "rv_map.cuh"
 #include "rv_whfast.cuh"
 #include "rv_rng.cuh"
 
@@ -49,6 +50,13 @@ struct rv_ctx {
     int* d_geo; size_t cap_geo;
     int* d_flag; size_t cap_flag;
     double* d_vhist; size_t cap_vhist;
+    // maximum-likelihood fit (rv_map_fit)
+    double* d_mrows; size_t cap_mrows;    // trial rows [running walkers][n_trial + 1][nvars]
+    double* d_mtlogp; size_t cap_mtlogp;
+    int* d_mtstat; size_t cap_mtstat;
+    double* d_mmu; size_t cap_mmu;        // per-walker damping
+    int* d_mfit; size_t cap_mfit;         // fit code[W], n_iter[W]
+    int* d_mlist; size_t cap_mlist;       // running list, next running list, evaluation list [W] each; counts[2]
     char err[512];
 };
 struct rv_obs {
@@ -168,6 +176,7 @@ int rv_ctx_destroy(rv_ctx* c) {
     cudaFree(c->d_chain); cudaFree(c->d_chainlp); cudaFree(c->d_nacc); cudaFree(c->d_acc);
     cudaFree(c->d_vpart); cudaFree(c->d_grad); cudaFree(c->d_hess);
     cudaFree(c->d_pgrad); cudaFree(c->d_phess); cudaFree(c->d_qf); cudaFree(c->d_lascr); cudaFree(c->d_geo); cudaFree(c->d_flag); cudaFree(c->d_vhist);
+    cudaFree(c->d_mrows); cudaFree(c->d_mtlogp); cudaFree(c->d_mtstat); cudaFree(c->d_mmu); cudaFree(c->d_mfit); cudaFree(c->d_mlist);
     cudaStreamDestroy(c->stream);
     delete c;
     return 0;
@@ -403,11 +412,8 @@ int rv_initial_conditions(rv_ctx* ctx, const rv_model* model, const double* thet
 // ------------------------------------------------------------------------------------------------
 // value + gradient + Hessian
 
-// check_prior is a per-call argument: the samplers always test priorHard (mcmc.py:171), whatever the model option says;
-// the plain entry points follow the model option (default 1), rv_loglik_d_dd_opt takes it from the caller.
-static int var_dev_impl(rv_ctx* ctx, const rv_model* model, const rv_obs* obs, const double* d_theta, int64_t W,
-                        double* d_logp, double* d_grad, double* d_hess, int32_t* d_status, int check_prior, cudaStream_t s) {
-    if (W == 0) return 0;
+// 0 when launch_var has a configuration for this model, else -31 (WHFast) or -30 (too many planets / parameters)
+static int var_refusal(rv_ctx* ctx, const rv_model* model) {
     const int nv = model->h.nvars;
     if (model->h.integrator != 0)
         return fail(ctx, -31, "the variational (gradient + Hessian) path integrates with IAS15 only; set integrator = 0");
@@ -421,6 +427,16 @@ static int var_dev_impl(rv_ctx* ctx, const rv_model* model, const rv_obs* obs, c
     if (!set_per_lane && !rv::var_model_fits(model->h.P, model->h.D, nv))
         return fail(ctx, -30, "variational kernel: %d planets x %d free parameters: the real and first-order sets alone need %d threads of one block",
                     model->h.P, nv, (nv + 1) * model->h.P);
+    return 0;
+}
+
+// check_prior is a per-call argument: the samplers always test priorHard (mcmc.py:171), whatever the model option says;
+// the plain entry points follow the model option (default 1), rv_loglik_d_dd_opt takes it from the caller.
+static int var_dev_impl(rv_ctx* ctx, const rv_model* model, const rv_obs* obs, const double* d_theta, int64_t W,
+                        double* d_logp, double* d_grad, double* d_hess, int32_t* d_status, int check_prior, cudaStream_t s) {
+    if (W == 0) return 0;
+    if (int rc = var_refusal(ctx, model)) return rc;
+    const int nv = model->h.nvars;
     const int nsets = rv::var_nsets(nv);
     if (int rc = ensure(ctx, &ctx->d_vpart, &ctx->cap_vpart, (size_t)(2 * W) * nsets)) return rc;
     if (int rc = ensure(ctx, &ctx->d_pstat, &ctx->cap_pstat, (size_t)(2 * W))) return rc;
@@ -478,6 +494,96 @@ int rv_loglik_d_dd_opt(rv_ctx* ctx, const rv_model* model, const rv_obs* obs, co
         CU(ctx, cudaMemcpyAsync(grad, ctx->d_grad, (size_t)W * nv * sizeof(double), cudaMemcpyDeviceToHost, s));
         CU(ctx, cudaMemcpyAsync(hess, ctx->d_hess, (size_t)W * nv * nv * sizeof(double), cudaMemcpyDeviceToHost, s));
     }
+    CU(ctx, cudaStreamSynchronize(s));
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// maximum-likelihood fit: damped saddle-free Newton per walker, batched line search (DESIGN.md 3.6)
+
+// One iteration: (1) the variational evaluation of the walkers whose theta moved (or that are new), gathered into one
+// contiguous batch and scattered back; (2) the Newton step of every running walker, n_trial + 1 rows each; (3) one plain
+// likelihood launch over all rows; (4) selection + compaction into the next running / evaluation lists.  The host reads
+// the two list lengths once per iteration; the loop ends when no walker runs.
+static int map_fit_impl(rv_ctx* ctx, const rv_model* model, const rv_obs* obs, int64_t W, int max_iter, int n_trial,
+                        double tol, double damping0, cudaStream_t s) {
+    const int nv = model->h.nvars;
+    const size_t nvs = (size_t)nv, R = (size_t)n_trial + 1;
+    if (int rc = ensure(ctx, &ctx->d_prop, &ctx->cap_prop, (size_t)W * nvs)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_plogp, &ctx->cap_plogp, (size_t)W)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_pstatus, &ctx->cap_pstatus, (size_t)W)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_pgrad, &ctx->cap_pgrad, (size_t)W * nvs)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_phess, &ctx->cap_phess, (size_t)W * nvs * nvs)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_lascr, &ctx->cap_lascr, (size_t)W * 2 * nvs * nvs)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_mrows, &ctx->cap_mrows, (size_t)W * R * nvs)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_mtlogp, &ctx->cap_mtlogp, (size_t)W * R)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_mtstat, &ctx->cap_mtstat, (size_t)W * R)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_mmu, &ctx->cap_mmu, (size_t)W)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_mfit, &ctx->cap_mfit, (size_t)2 * W)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_mlist, &ctx->cap_mlist, (size_t)3 * W + 2)) return rc;
+    int* code = ctx->d_mfit;
+    int* iters = ctx->d_mfit + W;
+    int* run = ctx->d_mlist;
+    int* run_next = ctx->d_mlist + W;
+    int* eval = ctx->d_mlist + 2 * W;
+    int* counts = ctx->d_mlist + 3 * W;
+    CU(ctx, rv::launch_map_init(W, damping0, code, iters, ctx->d_mmu, run, eval, s));
+    long long n_run = W, n_eval = W;
+    while (n_run > 0) {
+        if (n_eval > 0) {
+            CU(ctx, rv::launch_map_gather(eval, n_eval, ctx->d_theta, nv, ctx->d_prop, s));
+            if (int rc = var_dev_impl(ctx, model, obs, ctx->d_prop, n_eval, ctx->d_plogp, ctx->d_pgrad, ctx->d_phess,
+                                      ctx->d_pstatus, 1, s)) return rc;
+            CU(ctx, rv::launch_map_scatter(eval, n_eval, nv, ctx->d_plogp, ctx->d_pgrad, ctx->d_phess, ctx->d_pstatus,
+                                           ctx->d_logp, ctx->d_grad, ctx->d_hess, ctx->d_status, code, iters, s));
+        }
+        CU(ctx, rv::launch_map_step(run, n_run, nv, ctx->d_theta, ctx->d_grad, ctx->d_hess, ctx->d_mmu, iters, code, max_iter,
+                                    tol, n_trial, ctx->d_mrows, ctx->d_lascr, s));
+        if (int rc = loglik_dev_impl(ctx, model, obs, ctx->d_mrows, n_run * (int64_t)R, ctx->d_mtlogp, ctx->d_mtstat, s)) return rc;
+        CU(ctx, cudaMemsetAsync(counts, 0, 2 * sizeof(int), s));
+        CU(ctx, rv::launch_map_select(run, n_run, nv, n_trial, ctx->d_mrows, ctx->d_mtlogp, ctx->d_mtstat, ctx->d_theta,
+                                      ctx->d_mmu, iters, code, run_next, eval, counts, s));
+        int h[2];
+        CU(ctx, cudaMemcpyAsync(h, counts, sizeof h, cudaMemcpyDeviceToHost, s));
+        CU(ctx, cudaStreamSynchronize(s));
+        n_run = h[0]; n_eval = h[1];
+        int* t = run; run = run_next; run_next = t;
+    }
+    return 0;
+}
+
+int rv_map_fit(rv_ctx* ctx, const rv_model* model, const rv_obs* obs, double* theta, int64_t W, int max_iter, int n_trial,
+               double tol, double damping0, double* logp, double* grad, double* hess, int32_t* status, int32_t* fit_code,
+               int32_t* n_iter) {
+    if (!ctx || !model || !obs) return fail(ctx, -1, "rv_map_fit: NULL handle");
+    if (W < 0 || W >= ((int64_t)1 << 31)) return fail(ctx, -2, "rv_map_fit: W = %lld out of range [0, 2^31)", (long long)W);
+    if (n_trial < 1 || n_trial > rv::MAP_MAX_TRIAL)
+        return fail(ctx, -2, "rv_map_fit: n_trial = %d out of range 1..%d", n_trial, rv::MAP_MAX_TRIAL);
+    if (max_iter < 0) return fail(ctx, -2, "rv_map_fit: negative max_iter");
+    if (!(tol >= 0.0) || !(damping0 >= 0.0) || !isfinite(damping0))
+        return fail(ctx, -2, "rv_map_fit: tol and damping must be finite and >= 0");
+    const int nv = model->h.nvars;
+    if (nv < 1) return fail(ctx, -2, "rv_map_fit: the model has no free parameter");
+    if (int rc = var_refusal(ctx, model)) return rc;
+    if (W == 0) return 0;
+    if (!theta || !logp || !status || !fit_code || !n_iter) return fail(ctx, -1, "rv_map_fit: NULL buffer");
+    CU(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t s = ctx->stream;
+    const size_t nvs = (size_t)nv;
+    if (int rc = ensure(ctx, &ctx->d_theta, &ctx->cap_theta, (size_t)W * nvs)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_logp, &ctx->cap_logp, (size_t)W)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_status, &ctx->cap_status, (size_t)W)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_grad, &ctx->cap_grad, (size_t)W * nvs)) return rc;
+    if (int rc = ensure(ctx, &ctx->d_hess, &ctx->cap_hess, (size_t)W * nvs * nvs)) return rc;
+    CU(ctx, cudaMemcpyAsync(ctx->d_theta, theta, (size_t)W * nvs * sizeof(double), cudaMemcpyHostToDevice, s));
+    if (int rc = map_fit_impl(ctx, model, obs, W, max_iter, n_trial, tol, damping0, s)) return rc;
+    CU(ctx, cudaMemcpyAsync(theta, ctx->d_theta, (size_t)W * nvs * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CU(ctx, cudaMemcpyAsync(logp, ctx->d_logp, (size_t)W * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CU(ctx, cudaMemcpyAsync(status, ctx->d_status, (size_t)W * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CU(ctx, cudaMemcpyAsync(fit_code, ctx->d_mfit, (size_t)W * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CU(ctx, cudaMemcpyAsync(n_iter, ctx->d_mfit + W, (size_t)W * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    if (grad) CU(ctx, cudaMemcpyAsync(grad, ctx->d_grad, (size_t)W * nvs * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (hess) CU(ctx, cudaMemcpyAsync(hess, ctx->d_hess, (size_t)W * nvs * nvs * sizeof(double), cudaMemcpyDeviceToHost, s));
     CU(ctx, cudaStreamSynchronize(s));
     return 0;
 }

@@ -58,4 +58,16 @@ cudaError_t launch_stretch_accept_peer(const PeerCopies& pc, int self, long long
                                        unsigned long long id0_S, unsigned step, unsigned half, unsigned long long* n_accept,
                                        cudaStream_t s);
 cudaError_t launch_mask_logp(double* logp, const int* status, long long W, cudaStream_t s);
+// maximum-likelihood fit (rv_map.cu)
+cudaError_t launch_map_init(long long W, double mu0, int* code, int* n_iter, double* mu, int* run, int* eval, cudaStream_t s);
+cudaError_t launch_map_gather(const int* list, long long m, const double* theta, int n, double* out, cudaStream_t s);
+cudaError_t launch_map_scatter(const int* list, long long m, int n, const double* g_logp, const double* g_grad,
+                               const double* g_hess, const int* g_status, double* logp, double* grad, double* hess,
+                               int* status, int* code, const int* n_iter, cudaStream_t s);
+cudaError_t launch_map_step(const int* run, long long m, int n, const double* theta, const double* grad, const double* hess,
+                            const double* mu, const int* n_iter, int* code, int max_iter, double tol, int n_trial,
+                            double* rows, double* scratch, cudaStream_t s);
+cudaError_t launch_map_select(const int* run, long long m, int n, int n_trial, const double* rows, const double* tlogp,
+                              const int* tstatus, double* theta, double* mu, int* n_iter, int* code, int* run_next,
+                              int* eval, int* counts, cudaStream_t s);
 }  // namespace rv

@@ -4,13 +4,13 @@
 //   generate_proposal (:144-153)   Ginv = inv(G); L = cholesky(Ginv); mu = theta + eps^2 Ginv g / 2; theta* = mu + eps L z
 //   transitionProbability (:158-162)  log N(to; mu(from), eps^2 Ginv(from))
 //   step (:167-187)                accept iff exp(logp* - logp + q(theta|theta*) - q(theta*|theta)) > u
-// Nvars x Nvars (<= 21) linear algebra, one chain per thread: cyclic Jacobi, explicit G and G^-1, Cholesky.
+// Nvars x Nvars (<= 35) linear algebra, one chain per thread: cyclic Jacobi, explicit G and G^-1, Cholesky.
 #pragma once
 #include "rv_rng.cuh"
 
 namespace rv {
 
-constexpr int SMAX = MAXP_VAR * NELEM;   // 21: SMALA needs the variational kernels
+constexpr int SMAX = MAXP_VAR * NELEM;   // 35: SMALA needs the variational kernels
 
 // Cyclic Jacobi eigen-decomposition of the symmetric n x n matrix A (row-major, destroyed): A -> diag(lam), Q columns.
 RV_HD bool jacobi_eig(int n, double* A, double* Q, double* lam) {

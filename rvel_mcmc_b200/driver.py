@@ -197,6 +197,39 @@ def run_alsmala_gpu(label, Niter, true_state, obs, eps, alpha, bern_a, bern_b=No
     return _bundle_from_device("alsmala", r, "chain_logp", true_state, obs, Niter * nchains, nchains, label, t0)
 
 
+def find_map_gpu(true_state, obs, nstarts, scal, width=1.0, seed=0, **kw):
+    """Multi-start maximum-likelihood fit (ModelHandle.map_fit; keyword arguments max_iter, n_trial, tol, damping) from the
+    ball true_state + width*scales*N(0,1), drawn from np.random.default_rng(seed).  Not in the reference.
+
+    Returns dict(results, maxima).  results: the per-start arrays of map_fit plus `start`, sorted by logp (highest first).
+    maxima: the distinct converged maxima, highest first; converged starts are grouped greedily in that order -- a start
+    joins the first group whose best point it lies within 0.1 Laplace sigma of in every coordinate (that best point's
+    covariance) -- and each maximum is dict(state, theta, logp, count, cov, sigma)."""
+    from . import _abi
+    ctx = _abi.default_context()
+    sc = _scale_vector(true_state, scal)
+    rng = np.random.default_rng(seed)
+    start = true_state.get_params()[None, :] + width * sc[None, :] * rng.normal(size=(nstarts, true_state.Nvars))
+    r = true_state._model(ctx).map_fit(obs._handle(ctx), start, **kw)
+    r["start"] = start
+    order = np.argsort(-r["logp"], kind="stable")
+    results = {k: v[order] for k, v in r.items()}
+    maxima = []
+    for w in range(nstarts):
+        if results["fit_code"][w] != _abi.RV_FIT_CONVERGED:
+            continue
+        th = results["theta"][w]
+        for g in maxima:
+            if np.all(np.abs(th - g["theta"]) <= 0.1 * g["sigma"]):
+                g["count"] += 1
+                break
+        else:
+            st = true_state._fitted(results, w)
+            cov = st.laplace_cov
+            maxima.append(dict(state=st, theta=th, logp=st.logp, count=1, cov=cov, sigma=np.sqrt(np.diag(cov))))
+    return dict(results=results, maxima=maxima)
+
+
 def create_obs(state, npoint, err, errVar, t):
     return observations.FakeObservation(state, Npoints=npoint, error=err, errorVar=errVar, tmax=t)
 

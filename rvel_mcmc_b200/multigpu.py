@@ -64,6 +64,13 @@ class DeviceGroup(object):
         parts = self._map(len(theta), lambda r, lo, hi: hs[r][0].loglik_d_dd(hs[r][1], theta[lo:hi]))
         return tuple(np.concatenate([p[k] for p in parts]) for k in range(4))
 
+    def map_fit(self, state, obs, theta, **kw):
+        """ModelHandle.map_fit with the starts sharded over the GPUs (every walker's fit is independent)."""
+        theta = np.ascontiguousarray(theta, dtype=np.float64)
+        hs = self._handles(state, obs)
+        parts = self._map(len(theta), lambda r, lo, hi: hs[r][0].map_fit(hs[r][1], theta[lo:hi], **kw))
+        return {k: np.concatenate([p[k] for p in parts]) for k in parts[0]}
+
     # ---- independent chains -------------------------------------------------------------------------------------
     @staticmethod
     def _merge(parts):

@@ -290,6 +290,31 @@ class State(object):
             self.logp, self.logp_d, self.logp_dd = -chi, -chi_d, -chi_dd
         return self.logp, self.logp_d, self.logp_dd
 
+    def find_map(self, obs, **kw):
+        """Maximum-likelihood fit started at this state (ModelHandle.map_fit; keyword arguments max_iter, n_trial, tol,
+        damping).  Not in the reference.  Returns a new State at the optimum with logp / logp_d / logp_dd cached, `fit_code`
+        (RV_FIT_*) and `laplace_cov` (-inv(logp_dd) when the fit converged, else None).  Like get_logp, the evaluation keeps
+        this state's hillRadiusFactor.  Raises Encounter / RvGpuError when the start itself does not evaluate."""
+        ctx = _abi.default_context()
+        r = self._model(ctx).map_fit(obs._handle(ctx), self.get_params()[None, :], **kw)
+        if r["fit_code"][0] == _abi.RV_FIT_NOSTART:
+            if r["status"][0] == _abi.RV_ENCOUNTER:
+                raise Encounter("Two particles had a close encounter (d<exit_min_distance).")
+            raise _abi.RvGpuError("the fit's start does not evaluate (status %d)" % r["status"][0])
+        return self._fitted(r, 0)
+
+    def _fitted(self, r, w):
+        """New State at walker w of a map_fit result, with this state's hillRadiusFactor (the fit is an evaluation like
+        get_logp, not a sampler, so deepcopy's reset to 1 does not apply)."""
+        st = self.deepcopy()
+        st.hillRadiusFactor = self.hillRadiusFactor
+        st.set_params(r["theta"][w])
+        st.logp, st.logp_d, st.logp_dd = float(r["logp"][w]), r["grad"][w].copy(), r["hess"][w].copy()
+        st.fit_code = int(r["fit_code"][w])
+        st.n_iter = int(r["n_iter"][w])
+        st.laplace_cov = np.linalg.inv(-st.logp_dd) if st.fit_code == _abi.RV_FIT_CONVERGED else None
+        return st
+
     def priorHard(self):
         """state.py:299-315."""
         for i, planet in enumerate(self.planets):
