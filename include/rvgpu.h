@@ -89,8 +89,6 @@ int rv_model_destroy(rv_model* model);
 /* options: "integrator" (0 = IAS15, rebound's default and what the reference runs; 1 = WHFast, fixed step "dt0", each leg
  *   swept monotonically -- no reference call site, parity unpinned; rv_loglik_d_dd / rv_smala_run refuse it),
  * "dt0" (1e-3), "epsilon" (1e-9), "max_attempts", "hill_factor", "mapping" (0 lane-per-planet, 1 thread-per-walker),
- * "var_layout" (variational kernel: 0 = one lane per variational set where available (one or two planets), 1 = one
- *   thread per (set, planet)),
  * "check_prior" (1; 0 = rv_loglik_d_dd / rv_loglik_d_dd_dev integrate even outside the hard prior, as state.py:290
  *   does; the samplers ignore it and always test the prior; prefer rv_loglik_d_dd_opt's per-call argument),
  * "monotone_backward" (0 = rv_loglik visits obs.tb in its stored order as state.py:91 does; 1 = one sweep from 0 to the

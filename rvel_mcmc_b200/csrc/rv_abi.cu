@@ -70,7 +70,6 @@ struct rv_model {
     rv::Model h;
     rv::Model* d;
     int mapping;
-    int var_layout;    // 0 automatic, 1 thread per (set, planet) -- see launch_var
     int cost_order;    // 1 (default): the likelihood kernel takes its items most expensive first (launch_cost_order)
 };
 
@@ -229,7 +228,7 @@ int rv_model_create(rv_ctx* ctx, int n_planets, const double* fixed, int nvars, 
     if (!ctx || !out || !fixed) return fail(ctx, -1, "rv_model_create: NULL argument");
     rv_model* m = new (std::nothrow) rv_model();
     if (!m) return fail(ctx, -12, "out of host memory");
-    m->ctx = ctx; m->mapping = 0; m->var_layout = 0; m->cost_order = 1; m->d = nullptr;
+    m->ctx = ctx; m->mapping = 0; m->cost_order = 1; m->d = nullptr;
     const int rc = rv::build_model(&m->h, n_planets, fixed, nvars, free_planet, free_elem, hill_factor, dims);
     if (rc) {
         delete m;
@@ -259,7 +258,6 @@ int rv_model_set_option(rv_model* m, const char* key, double value) {
     else if (!strcmp(key, "max_attempts")) m->h.max_attempts = (int)value;
     else if (!strcmp(key, "hill_factor")) m->h.hill_factor = value;
     else if (!strcmp(key, "mapping")) m->mapping = (int)value;
-    else if (!strcmp(key, "var_layout")) m->var_layout = (int)value;
     else if (!strcmp(key, "cost_order")) m->cost_order = value != 0.0;
     else if (!strcmp(key, "check_prior")) m->h.check_prior = value != 0.0;
     else if (!strcmp(key, "monotone_backward")) m->h.monotone_backward = value != 0.0;
@@ -423,8 +421,7 @@ static int var_refusal(rv_ctx* ctx, const rv_model* model) {
     // models whose (set, planet) threads do not fit one CTA run their second-order sets in chunks (launch_var_chunked); what must
     // fit is the real + first-order group beside at least one pair -- true for everything the schema allows (5 planets x 7 elements:
     // 180 threads of 320)
-    const bool set_per_lane = model->var_layout == 0 && model->h.P <= 2 && model->h.D == 2 && nv + 1 <= 32;
-    if (!set_per_lane && !rv::var_model_fits(model->h.P, model->h.D, nv))
+    if (!rv::var_model_fits(model->h.P, model->h.D, nv))
         return fail(ctx, -30, "variational kernel: %d planets x %d free parameters: the real and first-order sets alone need %d threads of one block",
                     model->h.P, nv, (nv + 1) * model->h.P);
     return 0;
@@ -449,10 +446,10 @@ static int var_dev_impl(rv_ctx* ctx, const rv_model* model, const rv_obs* obs, c
     a.part = ctx->d_vpart; a.part_status = ctx->d_pstat;
     a.item_counter = ctx->d_item_counter;
     a.work_counters = ctx->count_work ? ctx->d_work : nullptr;
-    const size_t nh = rv::var_hist_doubles_needed(model->h.P, model->h.D, nv, model->var_layout, ctx->num_sms);
+    const size_t nh = rv::var_hist_doubles_needed(model->h.P, model->h.D, nv, ctx->num_sms);
     if (nh) { if (int rc = ensure(ctx, &ctx->d_vhist, &ctx->cap_vhist, nh)) return rc; }
     a.hist = ctx->d_vhist; a.hist_doubles = ctx->cap_vhist;
-    CU(ctx, rv::launch_var(a, model->h.P, model->h.D, nv, model->var_layout, ctx->num_sms, s));
+    CU(ctx, rv::launch_var(a, model->h.P, model->h.D, nv, ctx->num_sms, s));
     CU(ctx, rv::launch_var_finalize(ctx->d_vpart, ctx->d_pstat, W, nv, d_logp, d_grad, d_hess, d_status, ctx->d_item_counter, s));
     return 0;
 }

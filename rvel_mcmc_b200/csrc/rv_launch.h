@@ -18,8 +18,8 @@ cudaError_t launch_cost_order(const Model* md, const double* theta, long long W,
 struct VarArgs;
 int var_threads_needed(int P, int nv);
 int var_model_fits(int P, int D, int nv);   // launch_var has a configuration for this model (one launch or chunks of pairs)
-size_t var_hist_doubles_needed(int P, int D, int nv, int layout, int num_sms);
-cudaError_t launch_var(const VarArgs& a, int P, int D, int nv, int layout, int num_sms, cudaStream_t stream);
+size_t var_hist_doubles_needed(int P, int D, int nv, int num_sms);
+cudaError_t launch_var(const VarArgs& a, int P, int D, int nv, int num_sms, cudaStream_t stream);
 cudaError_t launch_var_finalize(const double* part, const int* pstat, long long W, int nv, double* logp, double* grad,
                                 double* hess, int* status, unsigned long long* item_counter, cudaStream_t stream);
 // optional WHFast variant (rv_whfast_kernels.cu)

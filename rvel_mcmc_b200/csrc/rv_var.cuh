@@ -457,6 +457,191 @@ RV_D double var_star_vx(const double* __restrict__ vx, const double* __restrict_
 }
 
 // ---------------------------------------------------------------------------------------------
+// Step logic that does not depend on the thread layout: var_run_items below and var2_run_items (rv_var2.cuh) share it.
+
+// setup_sim, uniform part: the walker's elements; true when they violate the hard prior
+template <int P>
+RV_D bool var_item_setup(const Model* __restrict__ md, const double* __restrict__ theta, long long wi, int nv, double (&el)[P][NELEM]) {
+    bool bad = false;
+#pragma unroll
+    for (int i = 0; i < P; i++) {
+#pragma unroll
+        for (int k = 0; k < NELEM; k++) {
+            const int s = md->src[i * NELEM + k];
+            el[i][k] = (s >= 0) ? theta[wi * nv + s] : md->fixed[i * NELEM + k];
+        }
+        bad = bad || prior_hard(el[i]);
+    }
+    return bad;
+}
+
+// squared exit distance of the encounter test: (hill_factor x the largest Hill radius)^2
+template <int P>
+RV_D double var_exit_min2(const double (&el)[P][NELEM], double m0, double hill_factor) {
+    double hill = 0.0;
+#pragma unroll
+    for (int i = 0; i < P; i++) {
+        const double rh = el[i][EL_A] * pow(el[i][EL_M] / (3.0 * m0), 1.0 / 3.0);
+        if (rh > hill) hill = rh;
+    }
+    const double emd = hill_factor * hill;
+    return emd * emd;
+}
+
+// g from b, in place (g_j needs b_k for k > j only), coordinate c
+template <int N>
+RV_D void var_g_from_b(double (&q)[7][N], int c) {
+#pragma unroll
+    for (int j = 0; j < 7; j++) {
+        double s = q[j][c];
+#pragma unroll
+        for (int k = 6; k > j; k--) s = fma(q[k][c], rvtab::DD[k][j], s);
+        q[j][c] = s;
+    }
+}
+
+// b from g, in place (b_k needs g_j for j > k only), coordinate c
+template <int N>
+RV_D void var_b_from_g(double (&q)[7][N], int c) {
+#pragma unroll
+    for (int k = 0; k < 7; k++) {
+        double s = q[k][c];
+#pragma unroll
+        for (int j = 6; j > k; j--) s = fma(q[j][c], rvtab::CC[j][k], s);
+        q[k][c] = s;
+    }
+}
+
+// rebound's step-size controller after an attempt of length dt, from the real particles' maxima of |b6| and |a|.  Sets the
+// next step in w.dt and returns true when the step is accepted; the caller then advances w.t and w.dt_last_done by dt after
+// committing the coordinates (updating the clock here, before the commit, costs var2_kernel spill stores).
+RV_HD bool var_step_control(double maxb6, double maxak, double epsilon, VarClock& w, double dt) {
+    const double err = maxb6 / maxak;
+    double dt_new;
+    if (is_normal(err)) dt_new = inv_root7(err / epsilon) * dt;
+    else dt_new = dt * 4.0;
+    if (fabs(dt_new) < 0.25 * fabs(dt)) {
+        w.dt = dt_new;
+        return false;
+    }
+    if (fabs(dt_new) > 4.0 * fabs(dt)) dt_new = dt * 4.0;
+    w.dt = dt_new;
+    return true;
+}
+
+// The per-coordinate step commit.  e(k, c): the coordinate's predicted e[k]; hist(k, c): the history of the last accepted
+// step, its e[k] at k < 7 and its b[k - 7] at k >= 7.  Rejected step: e and b re-predicted from the history, with
+// qr = new dt / that step's dt.
+template <int N, class E, class H>
+RV_D void var_reject_coord(double (&q)[7][N], int c, double qr, E&& e, H&& hist) {
+    double _e[7], _b[7], en[7];
+#pragma unroll
+    for (int k = 0; k < 7; k++) { _e[k] = hist(k, c); _b[k] = hist(7 + k, c); }
+    var_predict<N>(qr, _e, _b, en, q, c);
+#pragma unroll
+    for (int k = 0; k < 7; k++) e(k, c) = en[k];
+}
+
+// Accepted step of length dt (dt2 = dt^2): x0 and v0 advance with compensated summation (carries csx, csv), e and b become
+// the history, and the next step's e and b are predicted with qr = new dt / dt.
+template <int N, class E, class H>
+RV_D void var_accept_coord(double (&q)[7][N], int c, double& x0, double& csx, double& v0, double& csv, const double& a0,
+                           double dt, double dt2, double qr, E&& e, H&& hist) {
+    {
+        const double x = x0;
+        double cs = csx;
+        double s = q[6][c] * (1. / 72.);
+        s = fma(q[5][c], 1. / 56., s); s = fma(q[4][c], 1. / 42., s); s = fma(q[3][c], 1. / 30., s);
+        s = fma(q[2][c], 1. / 20., s); s = fma(q[1][c], 1. / 12., s); s = fma(q[0][c], 1. / 6., s);
+        s = fma(a0, 0.5, s);
+        cs += fma(s, dt2, v0 * dt);
+        const double xnew = x + cs;
+        cs += x - xnew;
+        x0 = xnew; csx = cs;
+    }
+    {
+        const double v = v0;
+        double cs = csv;
+        double s = q[6][c] * (1. / 8.);
+        s = fma(q[5][c], 1. / 7., s); s = fma(q[4][c], 1. / 6., s); s = fma(q[3][c], 1. / 5., s);
+        s = fma(q[2][c], 1. / 4., s); s = fma(q[1][c], 1. / 3., s); s = fma(q[0][c], 1. / 2., s);
+        s += a0;
+        cs = fma(s, dt, cs);
+        const double vnew = v + cs;
+        cs += v - vnew;
+        v0 = vnew; csv = cs;
+    }
+    double _e[7], _b[7], en[7];
+#pragma unroll
+    for (int k = 0; k < 7; k++) {
+        _e[k] = e(k, c);
+        _b[k] = q[k][c];
+        hist(k, c) = _e[k];
+        hist(7 + k, c) = _b[k];
+    }
+    var_predict<N>(qr, _e, _b, en, q, c);
+#pragma unroll
+    for (int k = 0; k < 7; k++) e(k, c) = en[k];
+}
+
+// chi2 / d[a] / dd[a][b] term of one set at an epoch (state.py:264-271): res = star vx - observed RV, den = err^2 npoints.
+// order 0 real, 1 first-order set `set` of parameter pa, 2 second-order set `set` with first-order parents sa / sb (pa, pb).
+template <int P>
+RV_D double var_epoch_term(const double* __restrict__ vxs, const double* __restrict__ dm, const VarUniform<P>& u, int order,
+                           int set, int sa, int sb, int pa, int pb, double res, double den) {
+    if (order == 0) return res * res / den;
+    if (order == 1) {
+        const double da = var_star_vx<P>(vxs, dm, u, 1, set, 0, 0, pa, 0);
+        return 2. * da * res / den;
+    }
+    const double da = var_star_vx<P>(vxs, dm, u, 1, sa, 0, 0, pa, 0);
+    const double db = var_star_vx<P>(vxs, dm, u, 1, sb, 0, 0, pb, 0);
+    const double dab = var_star_vx<P>(vxs, dm, u, 2, set, sa, sb, pa, pb);
+    return 2. * dab * res / den + 2. * da * db / den;
+}
+
+// The reference's epoch loop (state.py:262-284) over the leg of `item`: forward in order, backward reversed.
+//   attempt()      one IAS15 step attempt of the whole CTA / group: bit 0 accepted, bit 1 encounter after the step
+//   encounter()    the encounter test on the current positions
+//   on_epoch(ie)   epoch ie reached: accumulate chi2 / d / dd; false when the star velocity is not finite
+// Returns the leg's status.
+template <class Exec, class Attempt, class Encounter, class OnEpoch>
+RV_D int var_leg_epochs(Exec& ex, const VarArgs& a, const Model* __restrict__ md, long long item, VarClock& w,
+                        Attempt&& attempt, Encounter&& encounter, OnEpoch&& on_epoch) {
+    const bool backward = item < a.W;
+    const int n = backward ? a.nb : a.nf;
+    const int base = backward ? a.nf : 0;
+    LegCursor c;
+    c.status = RUN; c.ie = 0; c.n = n; c.attempts = 0; c.tmax = 0.0; c.last_full_dt = 0.0; c.chi2 = 0.0;
+    int final_status = -1;
+    for (int ii = 0; ii < n && final_status < 0; ii++) {
+        const int ie = backward ? (base + n - 1 - ii) : (base + ii);
+        c.tmax = a.ot[ie];
+        c.last_full_dt = w.dt;
+        w.dt_last_done = 0.0;
+        c.status = RUN;
+        if (encounter()) c.status = ST_ENCOUNTER;
+        while (check_exit(w, c) < 0) {
+            int r;
+            bool dead = false;
+            for (;;) {
+                r = attempt();
+                c.attempts++;
+                if (c.attempts > md->max_attempts || !isfinite(w.dt) || w.dt == 0.0) { dead = true; break; }
+                if (r & 1) break;
+            }
+            if (dead) { c.status = ST_NONFINITE; break; }
+            if (r & 2) c.status = ST_ENCOUNTER;
+        }
+        w.dt = c.last_full_dt;
+        if (c.status != ST_OK) { final_status = c.status; break; }
+        if (!on_epoch(ie)) final_status = ST_NONFINITE;
+        ex.sync();
+    }
+    return final_status < 0 ? ST_OK : final_status;
+}
+
+// ---------------------------------------------------------------------------------------------
 // The CTA algorithm.  Exec provides:
 //   each(f)                  run f(VarThread&) for every thread of the CTA
 //   sync()                   CTA barrier
@@ -490,36 +675,15 @@ RV_D void var_run_items(Exec& ex, const VarArgs& a, const VarLayout& L, double* 
     for (;;) {
         const long long item = ex.fetch(a.item_counter);
         if (item >= n_items) break;
-        const bool backward = item < a.W;
-        const long long wi = backward ? item : item - a.W;
-        const int n = backward ? a.nb : a.nf;
-        const int base = backward ? a.nf : 0;
-        // ---- setup_sim (uniform part): elements, hard prior, masses, exit distance ----------------
+        const long long wi = item < a.W ? item : item - a.W;
         double el[P][NELEM];
-        bool bad = false;
-        double hill = 0.0;
-#pragma unroll
-        for (int i = 0; i < P; i++) {
-#pragma unroll
-            for (int k = 0; k < NELEM; k++) {
-                const int s = md->src[i * NELEM + k];
-                el[i][k] = (s >= 0) ? a.theta[wi * nv + s] : md->fixed[i * NELEM + k];
-            }
-            bad = bad || prior_hard(el[i]);
-            u.gm[i] = el[i][EL_M];
-            u.mu[i] = el[i][EL_M] / m0;
-        }
-        int final_status = -1;
+        const bool bad = var_item_setup<P>(md, a.theta, wi, nv, el);
+        int final_status = ST_PRIOR;
         unsigned long long n_force = 0, n_attempt = 0;
-        if (bad && a.check_prior) final_status = ST_PRIOR;
-        if (final_status < 0) {
+        if (!(bad && a.check_prior)) {
 #pragma unroll
-            for (int i = 0; i < P; i++) {
-                const double rh = el[i][EL_A] * pow(el[i][EL_M] / (3.0 * m0), 1.0 / 3.0);
-                if (rh > hill) hill = rh;
-            }
-            const double emd = md->hill_factor * hill;
-            u.min2 = emd * emd;
+            for (int i = 0; i < P; i++) { u.gm[i] = el[i][EL_M]; u.mu[i] = el[i][EL_M] / m0; }
+            u.min2 = var_exit_min2<P>(el, m0, md->hill_factor);
             int cur = 0;
             ex.each([&](VarThread<P, D>& th) {
                 if (th.order < 0) return;
@@ -543,8 +707,6 @@ RV_D void var_run_items(Exec& ex, const VarArgs& a, const VarLayout& L, double* 
 
             VarClock w;
             w.t = 0.0; w.dt = md->dt0; w.dt_last_done = 0.0;
-            LegCursor c;
-            c.status = RUN; c.ie = 0; c.n = n; c.attempts = 0; c.tmax = 0.0; c.last_full_dt = 0.0; c.chi2 = 0.0;
 
             // ---- one IAS15 step attempt of the whole CTA; bit0 accepted, bit1 encounter after the step ----
             auto attempt = [&]() -> int {
@@ -557,14 +719,7 @@ RV_D void var_run_items(Exec& ex, const VarArgs& a, const VarLayout& L, double* 
                     for (int cc = 0; cc < D; cc++) {
                         th.ha0[cc] = 0.5 * th.a0[cc];
                         th.x0c[cc] = th.x0[cc] - th.csx[cc];
-                        // g from b, in place (g_j needs b_k for k > j only)
-#pragma unroll
-                        for (int j = 0; j < 7; j++) {
-                            double s = th.q[j][cc];
-#pragma unroll
-                            for (int k = 6; k > j; k--) s = fma(th.q[k][cc], rvtab::DD[k][j], s);
-                            th.q[j][cc] = s;
-                        }
+                        var_g_from_b<D>(th.q, cc);
                     }
                 });
                 int buf = cur ^ 1;
@@ -603,20 +758,12 @@ RV_D void var_run_items(Exec& ex, const VarArgs& a, const VarLayout& L, double* 
                     n_force += 7;
                 }
                 n_force += 1;
-                // b from g, in place (b_k needs g_j for j > k only); then step-size control over the real particles
+                // b from g; then step-size control over the real particles
                 ex.each([&](VarThread<P, D>& th) {
                     double mb = 0.0, ma = 0.0;
                     if (th.order >= 0) {
 #pragma unroll
-                        for (int cc = 0; cc < D; cc++) {
-#pragma unroll
-                            for (int k = 0; k < 7; k++) {
-                                double s = th.q[k][cc];
-#pragma unroll
-                                for (int j = 6; j > k; j--) s = fma(th.q[j][cc], rvtab::CC[j][k], s);
-                                th.q[k][cc] = s;
-                            }
-                        }
+                        for (int cc = 0; cc < D; cc++) var_b_from_g<D>(th.q, cc);
                     }
                     if (th.order == 0) {
                         double v2 = 0.0, x2 = 0.0;
@@ -635,77 +782,30 @@ RV_D void var_run_items(Exec& ex, const VarArgs& a, const VarLayout& L, double* 
                 ex.sync();
                 double maxb6, maxak;
                 ex.read_max(maxb6, maxak);
-                const double err = maxb6 / maxak;
-                const double dt_done = dt;
-                double dt_new;
-                if (is_normal(err)) dt_new = inv_root7(err / u.epsilon) * dt_done;
-                else dt_new = dt_done * 4.0;
-                int result = 0;
-                if (fabs(dt_new) < 0.25 * fabs(dt_done)) {
-                    w.dt = dt_new;
+                const bool accepted = var_step_control(maxb6, maxak, u.epsilon, w, dt);
+                if (!accepted) {
                     if (w.dt_last_done != 0.0) {
                         const double q = w.dt / w.dt_last_done;
                         ex.each([&](VarThread<P, D>& th) {
                             if (th.order < 0) return;
+                            auto e = [&](int k, int c) -> double& { return esm[(k * D + c) * NT + th.tid]; };
+                            auto h = [&](int k, int c) -> double& { return hist[(k * D + c) * NT + th.tid]; };
 #pragma unroll
-                            for (int cc = 0; cc < D; cc++) {
-                                double _e[7], _b[7], e[7];
-#pragma unroll
-                                for (int k = 0; k < 7; k++) {
-                                    _e[k] = hist[(k * D + cc) * NT + th.tid];
-                                    _b[k] = hist[((7 + k) * D + cc) * NT + th.tid];
-                                }
-                                var_predict<D>(q, _e, _b, e, th.q, cc);
-#pragma unroll
-                                for (int k = 0; k < 7; k++) esm[(k * D + cc) * NT + th.tid] = e[k];
-                            }
+                            for (int cc = 0; cc < D; cc++) var_reject_coord<D>(th.q, cc, q, e, h);
                         });
                     }
                 } else {
-                    if (fabs(dt_new) > 4.0 * fabs(dt_done)) dt_new = dt_done * 4.0;
-                    w.dt = dt_new;
-                    const double dt2 = dt_done * dt_done;
-                    const double q = w.dt / dt_done;
+                    const double dt2 = dt * dt, q = w.dt / dt;
                     ex.each([&](VarThread<P, D>& th) {
                         if (th.order < 0) return;
+                        auto e = [&](int k, int c) -> double& { return esm[(k * D + c) * NT + th.tid]; };
+                        auto h = [&](int k, int c) -> double& { return hist[(k * D + c) * NT + th.tid]; };
 #pragma unroll
-                        for (int cc = 0; cc < D; cc++) {
-                            {
-                                const double x = th.x0[cc];
-                                double s = th.q[6][cc] * (1. / 72.);
-                                s = fma(th.q[5][cc], 1. / 56., s); s = fma(th.q[4][cc], 1. / 42., s); s = fma(th.q[3][cc], 1. / 30., s);
-                                s = fma(th.q[2][cc], 1. / 20., s); s = fma(th.q[1][cc], 1. / 12., s); s = fma(th.q[0][cc], 1. / 6., s);
-                                s = fma(th.a0[cc], 0.5, s);
-                                th.csx[cc] += fma(s, dt2, th.v0[cc] * dt_done);
-                                th.x0[cc] = x + th.csx[cc];
-                                th.csx[cc] += x - th.x0[cc];
-                            }
-                            {
-                                const double v = th.v0[cc];
-                                double s = th.q[6][cc] * (1. / 8.);
-                                s = fma(th.q[5][cc], 1. / 7., s); s = fma(th.q[4][cc], 1. / 6., s); s = fma(th.q[3][cc], 1. / 5., s);
-                                s = fma(th.q[2][cc], 1. / 4., s); s = fma(th.q[1][cc], 1. / 3., s); s = fma(th.q[0][cc], 1. / 2., s);
-                                s += th.a0[cc];
-                                th.csv[cc] = fma(s, dt_done, th.csv[cc]);
-                                th.v0[cc] = v + th.csv[cc];
-                                th.csv[cc] += v - th.v0[cc];
-                            }
-                            double _e[7], _b[7], e[7];
-#pragma unroll
-                            for (int k = 0; k < 7; k++) {
-                                _e[k] = esm[(k * D + cc) * NT + th.tid];
-                                _b[k] = th.q[k][cc];
-                                hist[(k * D + cc) * NT + th.tid] = _e[k];
-                                hist[((7 + k) * D + cc) * NT + th.tid] = _b[k];
-                            }
-                            var_predict<D>(q, _e, _b, e, th.q, cc);
-#pragma unroll
-                            for (int k = 0; k < 7; k++) esm[(k * D + cc) * NT + th.tid] = e[k];
-                        }
+                        for (int cc = 0; cc < D; cc++)
+                            var_accept_coord<D>(th.q, cc, th.x0[cc], th.csx[cc], th.v0[cc], th.csv[cc], th.a0[cc], dt, dt2, q, e, h);
                     });
-                    w.t += dt_done;
-                    w.dt_last_done = dt_done;
-                    result = 1;
+                    w.t += dt;
+                    w.dt_last_done = dt;
                 }
                 // publish x0 for the encounter test and the next attempt's a0
                 double* Xp = pos + cur * L.npos;
@@ -715,59 +815,25 @@ RV_D void var_run_items(Exec& ex, const VarArgs& a, const VarLayout& L, double* 
                     for (int cc = 0; cc < D; cc++) Xp[(th.set * P + th.planet) * D + cc] = th.x0[cc];
                 });
                 ex.sync();
-                if (var_encounter<P, D>(Xp, u)) result |= 2;
-                return result;
+                return (accepted ? 1 : 0) | (var_encounter<P, D>(Xp, u) ? 2 : 0);
             };
 
-            // ---- the reference's epoch loop (state.py:262-284): forward in order, backward reversed ----
-            for (int ii = 0; ii < n && final_status < 0; ii++) {
-                const int ie = backward ? (base + n - 1 - ii) : (base + ii);
-                c.tmax = a.ot[ie];
-                c.last_full_dt = w.dt;
-                w.dt_last_done = 0.0;
-                c.status = RUN;
-                if (var_encounter<P, D>(pos + cur * L.npos, u)) c.status = ST_ENCOUNTER;
-                while (check_exit(w, c) < 0) {
-                    int r;
-                    bool dead = false;
-                    for (;;) {
-                        r = attempt();
-                        c.attempts++;
-                        if (c.attempts > md->max_attempts || !isfinite(w.dt) || w.dt == 0.0) { dead = true; break; }
-                        if (r & 1) break;
-                    }
-                    if (dead) { c.status = ST_NONFINITE; break; }
-                    if (r & 2) c.status = ST_ENCOUNTER;
-                }
-                w.dt = c.last_full_dt;
-                if (c.status != ST_OK) { final_status = c.status; break; }
-                // epoch reached: star vx of every set, chi2 / d / dd sums (state.py:264-271)
-                ex.each([&](VarThread<P, D>& th) { if (th.order >= 0) vxs[th.set * P + th.planet] = th.v0[0]; });
-                ex.sync();
-                const double svx = var_star_vx<P>(vxs, dm, u, 0, 0, 0, 0, 0, 0);
-                if (!isfinite(svx)) {
-                    final_status = ST_NONFINITE;
-                } else {
+            final_status = var_leg_epochs(ex, a, md, item, w, attempt,
+                [&]() { return var_encounter<P, D>(pos + cur * L.npos, u); },
+                [&](int ie) {
+                    // star vx of every set, chi2 / d / dd sums (state.py:264-271)
+                    ex.each([&](VarThread<P, D>& th) { if (th.order >= 0) vxs[th.set * P + th.planet] = th.v0[0]; });
+                    ex.sync();
+                    const double svx = var_star_vx<P>(vxs, dm, u, 0, 0, 0, 0, 0, 0);
+                    if (!isfinite(svx)) return false;
                     const double res = svx - a.orv[ie], er = a.oerr[ie];
                     const double den = er * er * a.npoints;
                     ex.each([&](VarThread<P, D>& th) {
-                        if (th.order < 0 || th.planet != 0) return;
-                        if (th.order == 0) {
-                            th.acc += res * res / den;
-                        } else if (th.order == 1) {
-                            const double da = var_star_vx<P>(vxs, dm, u, 1, th.set, 0, 0, th.pa, 0);
-                            th.acc += 2. * da * res / den;
-                        } else {
-                            const double da = var_star_vx<P>(vxs, dm, u, 1, th.sa, 0, 0, th.pa, 0);
-                            const double db = var_star_vx<P>(vxs, dm, u, 1, th.sb, 0, 0, th.pb, 0);
-                            const double dab = var_star_vx<P>(vxs, dm, u, 2, th.set, th.sa, th.sb, th.pa, th.pb);
-                            th.acc += 2. * dab * res / den + 2. * da * db / den;
-                        }
+                        if (th.order >= 0 && th.planet == 0)
+                            th.acc += var_epoch_term<P>(vxs, dm, u, th.order, th.set, th.sa, th.sb, th.pa, th.pb, res, den);
                     });
-                }
-                ex.sync();
-            }
-            if (final_status < 0) final_status = ST_OK;
+                    return true;
+                });
         }
         // ---- results of this leg -----------------------------------------------------------------
         const int fs = final_status;

@@ -35,7 +35,7 @@ constexpr int VAR2_STATE_PER_COORD = 13;   // shared memory, per coordinate: x0,
 // one base pointer with compile-time offsets (no address arithmetic in the substep loop), and consecutive lanes' 8-byte
 // accesses fall into distinct bank pairs.
 RV_HD int var2_slot_stride(int D) { return (VAR2_STATE_PER_COORD * D) | 1; }
-constexpr int VAR2_HIST_PER_COORD = 14;    // global scratch (L2-resident), per coordinate: br[7], er[7] -- written once per
+constexpr int VAR2_HIST_PER_COORD = 14;    // global scratch (L2-resident), per coordinate: er[7], br[7] -- written once per
                                            // accepted step, read only when a step is rejected
 
 RV_HD int var2_min_threads(int nv) { return 32 * ((nv * (nv + 1) / 2 + 31) / 32 + 1); }
@@ -367,7 +367,7 @@ RV_D void var2_run_items(Exec& ex, const VarArgs& a, const Var2Layout& L, double
     constexpr int NC = P * D;
     const Model* __restrict__ md = a.model;
     const int nv = md->nvars;
-    const int NPS = L.nps, n2 = L.n2;
+    const int n2 = L.n2;
     double* const cbuf = sm + L.o_cbuf;
     double* const vxs = cbuf + L.cstride;          // the epoch exchange reuses the substep buffers (dead between steps)
     double* const dm = sm + L.o_dm;
@@ -381,14 +381,14 @@ RV_D void var2_run_items(Exec& ex, const VarArgs& a, const Var2Layout& L, double
     static_assert(sizeof(VarUniform<P>) <= 8 * sizeof(double), "VarUniform must fit its shared-memory slot");
     VarUniform<P>& u = *reinterpret_cast<VarUniform<P>*>(sm + L.o_uni);
     const double epsilon = md->epsilon;
-    // per-coordinate state: shared memory through var2_state(th, VK_*, c); the rejected-step history (k = 0..6 br, 7..13 er)
-    // in the group's global scratch with the same slot striding
+    // per-coordinate state: shared memory through var2_state(th, VK_*, c); the rejected-step history (k = 0..6 er, 7..13 br,
+    // as var_accept_coord stores it) in the group's global scratch with the same slot striding
     auto ST = [&](const Var2Thread<P, D>& th, int k, int c) -> double& { return var2_state(th, k, c); };
     auto HS = [&](const Var2Thread<P, D>& th, int k, int c) -> double& {
         const int p = c / D, d = c - p * D;
         return hist[(size_t)(th.slot0 + p * n2) * (VAR2_HIST_PER_COORD * D) + k * D + d];
     };
-    enum { K_X0 = VK_X0, K_CSX = VK_CSX, K_CSV = VK_CSV, K_X0C = VK_X0C, K_V0 = VK_V0, K_A0 = VK_A0, K_E = VK_E, H_BR = 0, H_ER = 7 };
+    enum { K_X0 = VK_X0, K_CSX = VK_CSX, K_CSV = VK_CSV, K_X0C = VK_X0C, K_V0 = VK_V0, K_A0 = VK_A0, K_E = VK_E };
     ex.each([&](Var2Thread<P, D>& th) { th.st = state; });
     // a lane's coordinate count: producer lanes carry one planet, so lanes the whole set
     auto NCOF = [](const Var2Thread<P, D>& th) { return th.role == 2 ? NC : D; };
@@ -404,36 +404,17 @@ RV_D void var2_run_items(Exec& ex, const VarArgs& a, const Var2Layout& L, double
     for (;;) {
         const long long item = ex.fetch(a.item_counter);
         if (item >= n_items) break;
-        const bool backward = item < a.W;
-        const long long wi = backward ? item : item - a.W;
-        const int n = backward ? a.nb : a.nf;
-        const int base = backward ? a.nf : 0;
+        const long long wi = item < a.W ? item : item - a.W;
         double el[P][NELEM];
-        bool bad = false;
-        double hill = 0.0;
-#pragma unroll
-        for (int i = 0; i < P; i++) {
-#pragma unroll
-            for (int k = 0; k < NELEM; k++) {
-                const int s = md->src[i * NELEM + k];
-                el[i][k] = (s >= 0) ? a.theta[wi * nv + s] : md->fixed[i * NELEM + k];
-            }
-            bad = bad || prior_hard(el[i]);
-        }
-        int final_status = -1;
+        const bool bad = var_item_setup<P>(md, a.theta, wi, nv, el);
+        int final_status = ST_PRIOR;
         unsigned long long n_force = 0, n_attempt = 0;
-        if (bad && a.check_prior) final_status = ST_PRIOR;
-        if (final_status < 0) {
-#pragma unroll
-            for (int i = 0; i < P; i++) {
-                const double rh = el[i][EL_A] * pow(el[i][EL_M] / (3.0 * m0), 1.0 / 3.0);
-                if (rh > hill) hill = rh;
-            }
-            const double emd = md->hill_factor * hill;
+        if (!(bad && a.check_prior)) {
+            const double min2 = var_exit_min2<P>(el, m0, md->hill_factor);
             ex.sync();                                  // nobody still reads the previous item's masses
 #pragma unroll
             for (int i = 0; i < P; i++) { u.gm[i] = el[i][EL_M]; u.mu[i] = el[i][EL_M] / m0; }
-            u.gm0 = m0; u.epsilon = epsilon; u.min2 = emd * emd;
+            u.gm0 = m0; u.epsilon = epsilon; u.min2 = min2;
             ex.sync();
 
             // Producer lanes publish their planet's position into buffer b (x0 or the predicted xn), and -- after a
@@ -493,7 +474,7 @@ RV_D void var2_run_items(Exec& ex, const VarArgs& a, const Var2Layout& L, double
                         ST(th, K_X0, c) = x0[c]; ST(th, K_CSX, c) = 0.0; ST(th, K_CSV, c) = 0.0;
                         ST(th, K_X0C, c) = x0[c]; ST(th, K_V0, c) = v0[c]; ST(th, K_A0, c) = 0.0;
 #pragma unroll
-                        for (int k = 0; k < 7; k++) { ST(th, K_E + k, c) = 0.0; HS(th, H_BR + k, c) = 0.0; HS(th, H_ER + k, c) = 0.0; }
+                        for (int k = 0; k < 7; k++) { ST(th, K_E + k, c) = 0.0; HS(th, k, c) = 0.0; HS(th, 7 + k, c) = 0.0; }
                     }
                 }
             });
@@ -502,8 +483,6 @@ RV_D void var2_run_items(Exec& ex, const VarArgs& a, const Var2Layout& L, double
 
             VarClock w;
             w.t = 0.0; w.dt = md->dt0; w.dt_last_done = 0.0;
-            LegCursor c;
-            c.status = RUN; c.ie = 0; c.n = n; c.attempts = 0; c.tmax = 0.0; c.last_full_dt = 0.0; c.chi2 = 0.0;
 
             // ---- one IAS15 step attempt of the whole group; bit0 accepted, bit1 encounter after the step ----
             auto attempt = [&]() -> int {
@@ -521,13 +500,7 @@ RV_D void var2_run_items(Exec& ex, const VarArgs& a, const Var2Layout& L, double
                         if (cc >= nc) break;
                         ST(th, K_A0, cc) = a0[cc];
                         ST(th, K_X0C, cc) = x0[cc] - ST(th, K_CSX, cc);
-#pragma unroll
-                        for (int j = 0; j < 7; j++) {      // g from b, in place
-                            double s = th.q[j][cc];
-#pragma unroll
-                            for (int k = 6; k > j; k--) s = fma(th.q[k][cc], rvtab::DD[k][j], s);
-                            th.q[j][cc] = s;
-                        }
+                        var_g_from_b<NC>(th.q, cc);
                     }
                 });
                 Ratio pc_err{1e300, 1.0}, pc_last{2.0, 1.0};
@@ -574,7 +547,7 @@ RV_D void var2_run_items(Exec& ex, const VarArgs& a, const Var2Layout& L, double
                     n_force += 7;
                 }
                 n_force += 1;
-                // b from g, in place; then step-size control over the real particles
+                // b from g; then step-size control over the real particles
                 ex.each([&](Var2Thread<P, D>& th) {
                     double mb = 0.0, ma = 0.0;
                     if (th.role >= 0) {
@@ -582,13 +555,7 @@ RV_D void var2_run_items(Exec& ex, const VarArgs& a, const Var2Layout& L, double
 #pragma unroll
                         for (int cc = 0; cc < NC; cc++) {
                             if (cc >= nc) break;
-#pragma unroll
-                            for (int k = 0; k < 7; k++) {
-                                double s = th.q[k][cc];
-#pragma unroll
-                                for (int j = 6; j > k; j--) s = fma(th.q[j][cc], rvtab::CC[j][k], s);
-                                th.q[k][cc] = s;
-                            }
+                            var_b_from_g<NC>(th.q, cc);
                         }
                     }
                     if (th.role == 0) {
@@ -608,147 +575,71 @@ RV_D void var2_run_items(Exec& ex, const VarArgs& a, const Var2Layout& L, double
                 ex.sync();
                 double maxb6, maxak;
                 ex.read_max(maxb6, maxak);
-                const double err = maxb6 / maxak;
-                const double dt_done = dt;
-                double dt_new;
-                if (is_normal(err)) dt_new = inv_root7(err / epsilon) * dt_done;
-                else dt_new = dt_done * 4.0;
-                int result = 0;
-                if (fabs(dt_new) < 0.25 * fabs(dt_done)) {
-                    w.dt = dt_new;
+                const bool accepted = var_step_control(maxb6, maxak, epsilon, w, dt);
+                if (!accepted) {
                     if (w.dt_last_done != 0.0) {
                         const double q = w.dt / w.dt_last_done;
                         ex.each([&](Var2Thread<P, D>& th) {
                             if (th.role < 0) return;
                             const int nc = NCOF(th);
+                            auto e = [&](int k, int c) -> double& { return ST(th, K_E + k, c); };
+                            auto h = [&](int k, int c) -> double& { return HS(th, k, c); };
 #pragma unroll
                             for (int cc = 0; cc < NC; cc++) {
                                 if (cc >= nc) break;
-                                double _e[7], _b[7], e[7];
-#pragma unroll
-                                for (int k = 0; k < 7; k++) { _e[k] = HS(th, H_ER + k, cc); _b[k] = HS(th, H_BR + k, cc); }
-                                var_predict<NC>(q, _e, _b, e, th.q, cc);
-#pragma unroll
-                                for (int k = 0; k < 7; k++) ST(th, K_E + k, cc) = e[k];
+                                var_reject_coord<NC>(th.q, cc, q, e, h);
                             }
                         });
                     }
                 } else {
-                    if (fabs(dt_new) > 4.0 * fabs(dt_done)) dt_new = dt_done * 4.0;
-                    w.dt = dt_new;
-                    const double dt2 = dt_done * dt_done;
-                    const double q = w.dt / dt_done;
+                    const double dt2 = dt * dt, q = w.dt / dt;
                     ex.each([&](Var2Thread<P, D>& th) {
                         if (th.role < 0) return;
                         const int nc = NCOF(th);
+                        auto e = [&](int k, int c) -> double& { return ST(th, K_E + k, c); };
+                        auto h = [&](int k, int c) -> double& { return HS(th, k, c); };
 #pragma unroll
                         for (int cc = 0; cc < NC; cc++) {
                             if (cc >= nc) break;
-                            {
-                                const double x = ST(th, K_X0, cc);
-                                double csx = ST(th, K_CSX, cc);
-                                double s = th.q[6][cc] * (1. / 72.);
-                                s = fma(th.q[5][cc], 1. / 56., s); s = fma(th.q[4][cc], 1. / 42., s); s = fma(th.q[3][cc], 1. / 30., s);
-                                s = fma(th.q[2][cc], 1. / 20., s); s = fma(th.q[1][cc], 1. / 12., s); s = fma(th.q[0][cc], 1. / 6., s);
-                                s = fma(ST(th, K_A0, cc), 0.5, s);
-                                csx += fma(s, dt2, ST(th, K_V0, cc) * dt_done);
-                                const double xnew = x + csx;
-                                csx += x - xnew;
-                                ST(th, K_X0, cc) = xnew; ST(th, K_CSX, cc) = csx;
-                            }
-                            {
-                                const double v = ST(th, K_V0, cc);
-                                double csv = ST(th, K_CSV, cc);
-                                double s = th.q[6][cc] * (1. / 8.);
-                                s = fma(th.q[5][cc], 1. / 7., s); s = fma(th.q[4][cc], 1. / 6., s); s = fma(th.q[3][cc], 1. / 5., s);
-                                s = fma(th.q[2][cc], 1. / 4., s); s = fma(th.q[1][cc], 1. / 3., s); s = fma(th.q[0][cc], 1. / 2., s);
-                                s += ST(th, K_A0, cc);
-                                csv = fma(s, dt_done, csv);
-                                const double vnew = v + csv;
-                                csv += v - vnew;
-                                ST(th, K_V0, cc) = vnew; ST(th, K_CSV, cc) = csv;
-                            }
-                            double _e[7], _b[7], e[7];
-#pragma unroll
-                            for (int k = 0; k < 7; k++) {
-                                _e[k] = ST(th, K_E + k, cc);
-                                _b[k] = th.q[k][cc];
-                                HS(th, H_ER + k, cc) = _e[k];
-                                HS(th, H_BR + k, cc) = _b[k];
-                            }
-                            var_predict<NC>(q, _e, _b, e, th.q, cc);
-#pragma unroll
-                            for (int k = 0; k < 7; k++) ST(th, K_E + k, cc) = e[k];
+                            var_accept_coord<NC>(th.q, cc, ST(th, K_X0, cc), ST(th, K_CSX, cc), ST(th, K_V0, cc), ST(th, K_CSV, cc),
+                                                 ST(th, K_A0, cc), dt, dt2, q, e, h);
                         }
                     });
-                    w.t += dt_done;
-                    w.dt_last_done = dt_done;
-                    result = 1;
+                    w.t += dt;
+                    w.dt_last_done = dt;
                 }
                 // publish x0 of the producer sets for the encounter test and the next attempt's a0
                 publish_positions(0, false);
                 ex.sync();
+                int result = accepted ? 1 : 0;
                 if (var_encounter<P, D>(cbuf, u)) result |= 2;
                 return result;
             };
 
-            // ---- the reference's epoch loop (state.py:262-284): forward in order, backward reversed ----
-            for (int ii = 0; ii < n && final_status < 0; ii++) {
-                const int ie = backward ? (base + n - 1 - ii) : (base + ii);
-                c.tmax = a.ot[ie];
-                c.last_full_dt = w.dt;
-                w.dt_last_done = 0.0;
-                c.status = RUN;
-                if (var_encounter<P, D>(cbuf, u)) c.status = ST_ENCOUNTER;
-                while (check_exit(w, c) < 0) {
-                    int r;
-                    bool dead = false;
-                    for (;;) {
-                        r = attempt();
-                        c.attempts++;
-                        if (c.attempts > md->max_attempts || !isfinite(w.dt) || w.dt == 0.0) { dead = true; break; }
-                        if (r & 1) break;
-                    }
-                    if (dead) { c.status = ST_NONFINITE; break; }
-                    if (r & 2) c.status = ST_ENCOUNTER;
-                }
-                w.dt = c.last_full_dt;
-                if (c.status != ST_OK) { final_status = c.status; break; }
-                // epoch reached: star vx of every set, chi2 / d / dd sums (state.py:264-271)
-                ex.each([&](Var2Thread<P, D>& th) {
-                    if (th.role < 0) return;
-                    if (th.role == 2) {
+            final_status = var_leg_epochs(ex, a, md, item, w, attempt,
+                [&]() { return var_encounter<P, D>(cbuf, u); },
+                [&](int ie) {
+                    // star vx of every set, chi2 / d / dd sums (state.py:264-271)
+                    ex.each([&](Var2Thread<P, D>& th) {
+                        if (th.role < 0) return;
+                        if (th.role == 2) {
 #pragma unroll
-                        for (int p = 0; p < P; p++) vxs[th.set * P + p] = ST(th, K_V0, p * D);
-                    } else {
-                        vxs[th.set * P + th.planet] = ST(th, K_V0, 0);
-                    }
-                });
-                ex.sync();
-                const double svx = var_star_vx<P>(vxs, dm, u, 0, 0, 0, 0, 0, 0);
-                if (!isfinite(svx)) {
-                    final_status = ST_NONFINITE;
-                } else {
+                            for (int p = 0; p < P; p++) vxs[th.set * P + p] = ST(th, K_V0, p * D);
+                        } else {
+                            vxs[th.set * P + th.planet] = ST(th, K_V0, 0);
+                        }
+                    });
+                    ex.sync();
+                    const double svx = var_star_vx<P>(vxs, dm, u, 0, 0, 0, 0, 0, 0);
+                    if (!isfinite(svx)) return false;
                     const double res = svx - a.orv[ie], er = a.oerr[ie];
                     const double den = er * er * a.npoints;
                     ex.each([&](Var2Thread<P, D>& th) {
                         if (th.role < 0 || (th.role <= 1 && th.planet != 0)) return;
-                        if (th.role == 0) {
-                            th.acc += res * res / den;
-                        } else if (th.role == 1) {
-                            const double da = var_star_vx<P>(vxs, dm, u, 1, th.set, 0, 0, th.pa, 0);
-                            th.acc += 2. * da * res / den;
-                        } else {
-                            const double da = var_star_vx<P>(vxs, dm, u, 1, 1 + th.pa, 0, 0, th.pa, 0);
-                            const double db = var_star_vx<P>(vxs, dm, u, 1, 1 + th.pb, 0, 0, th.pb, 0);
-                            const double dab = var_star_vx<P>(vxs, dm, u, 2, th.set, 1 + th.pa, 1 + th.pb, th.pa, th.pb);
-                            th.acc += 2. * dab * res / den + 2. * da * db / den;
-                        }
+                        th.acc += var_epoch_term<P>(vxs, dm, u, th.role, th.set, 1 + th.pa, 1 + th.pb, th.pa, th.pb, res, den);
                     });
-                }
-                ex.sync();
-            }
-            if (final_status < 0) final_status = ST_OK;
+                    return true;
+                });
         }
         const int fs = final_status;
         ex.each([&](Var2Thread<P, D>& th) {

@@ -1,7 +1,8 @@
 // rv_var_kernels.cu -- sm_100a kernel for State.get_logp_d_dd (value + gradient + Hessian, SMALA).
 //
 // var_kernel: persistent grid; every CTA pulls (walker, leg) items and integrates the real system together
-// with its first- and second-order variational sets, one thread per (set, planet) -- see rv_var.cuh.
+// with its first- and second-order variational sets, one thread per (set, planet) -- see rv_var.cuh.  var2_kernel: the same
+// algorithm with one lane per second-order set, for one planet and two coplanar planets -- see rv_var2.cuh.
 #include <cuda_runtime.h>
 #include "rv_launch.h"
 #include "rv_var.cuh"
@@ -241,7 +242,7 @@ static cudaError_t launch_var_chunked(const VarArgs& a, int nv, int num_sms, cud
     return cudaSuccess;
 }
 
-// 1 when launch_var has a configuration for the thread-per-(set, planet) layout of this model (one launch or chunks)
+// 1 when launch_var has a configuration for this model (one or two planets: always; more: one launch or chunks of pairs)
 int var_model_fits(int P, int D, int nv) {
     if (P < 1 || P > MAXP_VAR) return 0;
     if (P <= 2) return 1;                                    // at most 14 free parameters: always one launch
@@ -255,27 +256,24 @@ int var_threads_needed(int P, int nv) {
 }
 
 // global history scratch (doubles) the warp-group kernel needs for this model on this GPU; 0 when the other layout runs
-size_t var_hist_doubles_needed(int P, int D, int nv, int layout, int num_sms) {
-    if (layout == 1 || !var2_supported(P, nv)) return 0;
+size_t var_hist_doubles_needed(int P, int D, int nv, int num_sms) {
+    if (!var2_supported(P, nv)) return 0;
     return (size_t)num_sms * 8 * var2_hist_doubles(P, D, nv);       // at most 8 resident groups per SM
 }
 
-// layout: 0 = automatic (warp-group kernel where it exists: one or two planets), 1 = thread per (set, planet)
-cudaError_t launch_var(const VarArgs& a, int P, int D, int nv, int layout, int num_sms, cudaStream_t stream) {
-    if (layout != 1 && var2_supported(P, nv)) {
+// One planet, or two coplanar planets: the warp-group kernel (a coplanar two-planet model has at most 10 free parameters and
+// a one-planet model at most 7, so 96 and 64 threads per group always suffice).  Two inclined planets and three to five
+// planets: one thread per (set, planet).
+cudaError_t launch_var(const VarArgs& a, int P, int D, int nv, int num_sms, cudaStream_t stream) {
+    if (var2_supported(P, nv)) {
         const int nt = var2_min_threads(nv);
         if (P == 2 && D == 2 && nt <= 96) {                       // nv <= 10 (HD155358): 4 x 96 = 384 threads, 168 registers
             if (var2_groups(2, 2, nv, 96, 4) >= 4) return launch_var2_one<2, 2, 96, 4, 168>(a, nv, num_sms, stream);
         }
-        // (a coplanar two-planet model has at most 10 free parameters, so 96 threads per group always suffice)
         if (P == 1 && D == 2 && nt <= 64) return launch_var2_one<1, 2, 64, 4, 128>(a, nv, num_sms, stream);
         if (P == 1 && D == 3 && nt <= 64) return launch_var2_one<1, 3, 64, 4, 168>(a, nv, num_sms, stream);
     }
     const int need = var_threads_needed(P, nv);
-    if (P == 1 && D == 2 && need <= 64) return launch_var_one<1, 2, 64, 4>(a, nv, num_sms, stream);
-    if (P == 1 && D == 3 && need <= 64) return launch_var_one<1, 3, 64, 4>(a, nv, num_sms, stream);
-    if (P == 2 && D == 2 && need <= 64) return launch_var_one<2, 2, 64, 4>(a, nv, num_sms, stream);
-    if (P == 2 && D == 2 && need <= 160) return launch_var_one<2, 2, 160, 3>(a, nv, num_sms, stream);
     if (P == 2 && D == 3 && need <= 256) return launch_var_one<2, 3, 256, 1>(a, nv, num_sms, stream);
     if (P == 3 && D == 2 && need <= 448) return launch_var_one<3, 2, 448, 1>(a, nv, num_sms, stream);
     // (inclined models: 320 threads -- the per-thread shared-memory history, 21 D doubles, is what fills the SM's 227 KB)
